@@ -1,8 +1,14 @@
 #!/usr/bin/env python
-"""Benchmark of the Raindrop hot path on B200 (driver contract: see the task statement).
+"""Benchmark of the Raindrop hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed TrainStep computed on rank 0 as float32
+DIR/<name>.npy: `loss`, `logits`, and per used parameter its updated value `param.<key>` and its gradient
+`grad.<key>` (state-dict keys).  Inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output.  Above 64 MiB in all, arrays larger than an even share are replaced by a fixed, seeded
+sample of their elements.
 
 A "step" is one training step of Raindrop_v2 (forward + CrossEntropy + backward + Adam, dropout 0.2,
 code/Raindrop.py:311-324) on one batch of synthetic data of the named configuration.  The default
@@ -10,7 +16,7 @@ configuration is the one BASELINE.json's metric is quoted on (configs[1]: P19 sh
 GPU, 34 sensors, T_max = 60); `--config` selects the other BASELINE configurations:
 
     P12      configs[0]  B = 32,  36 sensors, T = 215   (the reference's CPU-runnable case)
-    P19      configs[1]  B = 128, 34 sensors, T = 60    (default; the driver's line)
+    P19      configs[1]  B = 128, 34 sensors, T = 60    (default)
     PAM      configs[2]  B = 256, 17 sensors, T = 600, 8 classes, no static branch
     P19x4    configs[3]  B = 256 per GPU (1024 over 4 GPUs), leave-10-sensors-out mask
     LARGEx8  configs[4]  B = 512 per GPU (4096 over 8 GPUs), 128 sensors, T = 256
@@ -48,6 +54,7 @@ sys.path.insert(0, ROOT)
 
 import warnings  # noqa: E402
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 import torch.nn.functional as F  # noqa: E402
@@ -185,6 +192,23 @@ def summarize(per_step, world, device):
     return {"median": statistics.median(srt), "mean": sum(srt) / n, "p90": srt[min(n - 1, int(0.9 * n))],
             "max": srt[-1], "min": srt[0],
             "per_rank_median": [round(statistics.median(r), 4) for r in allt.cpu().tolist()]}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """name -> tensor, written as out_dir/<name>.npy in float32.  If they exceed DUMP_LIMIT_BYTES in all, every array
+    larger than an even share of the limit is replaced by that many elements at fixed, seeded positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // 4 // len(arrays)
+    over = sum(t.numel() for t in arrays.values()) * 4 > DUMP_LIMIT_BYTES
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if over and a.numel() > share:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def _round_tf32(t):
@@ -343,6 +367,7 @@ def main():
     ap.add_argument("--config", default="P19", choices=sorted(BENCH_CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -398,6 +423,12 @@ def main():
     ms_per_step = dev["median"]
     value = world * BATCH / (ms_per_step * 1e-3)
     loss_graph = float(ts.loss.item())
+    if args.dump_outputs and rank == 0:
+        outs = {"loss": ts.loss, "logits": ts.logits}
+        for (key, _), p, off in zip(ts.plan.fields, model.used_parameters(), ts.offsets):
+            outs["param." + key] = p.data
+            outs["grad." + key] = ts.flat_g[off:off + p.numel()].view(p.shape)
+        dump_outputs(args.dump_outputs, outs)
 
     # ---- leg 2: end to end through the drop-in module API, host batches ---------------------------
     model2 = build_model(cfg, device)

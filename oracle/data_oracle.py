@@ -9,7 +9,7 @@ Each function follows the reference line by line:
   remove_features        code/Raindrop.py:214-231
   epoch_batches          code/Raindrop.py:261-309  (strategy 2 and 3)
 Pinned against the reference's own functions in tests/test_data_pipeline.py::test_data_oracle_matches_reference
-(runs wherever /root/reference is present).
+(their outputs stored in tests/golden/data_pipeline.npz by oracle/make_golden.py).
 """
 import numpy as np
 import torch

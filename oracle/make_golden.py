@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by running the reference's own,
-unmodified files (oracle/ref_harness.py) on CPU in the build container:
+unmodified files (oracle/ref_harness.py) on CPU:
 
-    python -m oracle.make_golden            # from the repo root; needs /root/reference
+    RAINDROP_REFERENCE=<checkout of the original project> python -m oracle.make_golden [part]
 
 A fixture stores seeds + the reference's outputs; inputs and weights are regenerated from the
 seeds by raindrop_b200.synth (make_batch / synth_weights), so the files stay small.  Stored per
@@ -20,9 +20,10 @@ import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from oracle import ref_harness  # noqa: E402
-from raindrop_b200.synth import make_batch, model_config, synth_weights, used_param_keys  # noqa: E402
+from raindrop_b200.synth import keyed_values, make_batch, model_config, synth_weights, used_param_keys  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 N_SAMPLE = 509
@@ -198,38 +199,96 @@ def operator_grad_cases():
     print("operators_grad     %d arrays: %s" % (len(out), sorted(out)[:60]))
 
 
+V1_FULL_MAX = 4096      # v1 gradients with more elements are stored as fingerprints (keeps the file small)
+
+
 def v1_case():
     """Legacy `Raindrop` v1 (code/models_rd.py:46-191; hard-coded to 36 sensors / 215 steps): logits, loss and the
-    gradient of every parameter that gets one, B = 3, eval mode.  Weights: seeded default init, but `encoder` / `emb`
-    re-drawn at a useful scale (the reference initialises them to +-1e-10, which would hide the graph layer)."""
+    gradient of every parameter that gets one, B = 3, eval mode.  Weights: every state-dict entry from the keyed
+    stream (synth.keyed_values, weight seed 19), so the fixture stores no weights; `encoder` / `emb` thus get a useful
+    scale (the reference initialises them to +-1e-10, which would hide the graph layer)."""
     ref = ref_harness.load_reference()
     from raindrop_b200.synth import CONFIGS
     cfg = dict(CONFIGS["P12"]); cfg["name"] = "P12"
-    B = 3
+    B, wseed = 3, 19
     batch = make_batch(dict(cfg, d_ob=2), B, seed=77)
     torch.manual_seed(5)
     gs = (torch.rand(36, 36) < 0.5).float() * torch.rand(36, 36)
     model = ref.Raindrop(36, 72, 2, 144, 2, 0.2, 215, 9, 100, 0.5, "mean", 2, gs.clone()).eval()
-    with torch.no_grad():
-        model.encoder.weight.uniform_(-0.3, 0.3)
-        model.emb.weight.uniform_(-0.3, 0.3)
+    sd = model.state_dict()
+    model.load_state_dict({k: keyed_values(wseed, k, tuple(v.shape)) for k, v in sd.items()})
     logits, distance, _ = model.forward(batch["src"], batch["static"], batch["times"], batch["lengths"])
     loss = F.cross_entropy(logits, batch["y"])
     model.zero_grad()
     loss.backward()
     out = dict(logits=logits.detach().numpy(), loss=np.float32(loss.item()), distance=np.float32(float(distance)),
                global_structure=gs.numpy())
-    for k, v in model.state_dict().items():
-        out["sd." + k] = v.numpy()
-    for k, prm in model.named_parameters():
-        if prm.grad is not None:
-            out["grad." + k] = prm.grad.numpy()
-    meta = dict(case="v1_p12_b3", batch=B, data_seed=77, torch=torch.__version__, reference_commit="892eb57",
-                generator="oracle/make_golden.py v1")
+    with_grad = [k for k, prm in model.named_parameters() if prm.grad is not None]
+    for k in with_grad:
+        g = model.get_parameter(k).grad
+        if g.numel() <= V1_FULL_MAX:
+            out["grad." + k] = g.numpy()
+        else:
+            fp = fingerprint(g)
+            out["grad." + k + "#sample"] = fp["sample"]
+            out["grad." + k + "#stats"] = np.array([fp["sum"], fp["asum"], fp["l2"]], dtype=np.float64)
+    meta = dict(case="v1_p12_b3", batch=B, data_seed=77, weight_seed=wseed, torch=torch.__version__,
+                reference_commit="892eb57", generator="oracle/make_golden.py v1",
+                state_dict={k: list(v.shape) for k, v in sd.items()}, with_grad=with_grad)
     out["meta"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
     np.savez_compressed(os.path.join(GOLDEN, "v1_p12_b3.npz"), **out)
     print("v1_p12_b3  logits[0]=%s loss=%.6f distance=%g grads for %d tensors" %
-          (logits[0].tolist(), loss.item(), float(distance), sum(1 for k in out if k.startswith("grad."))))
+          (logits[0].tolist(), loss.item(), float(distance), len(with_grad)))
+
+
+def default_init_case():
+    """The reference's Raindrop_v2 as code/Raindrop.py:245-251 constructs it (torch.manual_seed(1), the modules' own
+    initialisation, TINY shape): its state dict (entries above 1024 elements as fingerprints) and its eval-mode
+    logits on make_batch(seed=1)."""
+    cfg = model_config("TINY", dropout=0.2)
+    ref = ref_harness.build_reference_model(cfg).eval()
+    batch = make_batch(cfg, 3, seed=1)
+    with torch.no_grad():
+        logits = ref.forward(batch["src"], batch["static"], batch["times"], batch["lengths"])[0]
+    out = {"logits": logits.numpy()}
+    sd = ref.state_dict()
+    for k, v in sd.items():
+        if v.numel() <= 1024:
+            out["sd." + k] = v.numpy()
+        else:
+            fp = fingerprint(v)
+            out["sd." + k + "#sample"] = fp["sample"]
+            out["sd." + k + "#stats"] = np.array([fp["sum"], fp["asum"], fp["l2"]], dtype=np.float64)
+    out["meta"] = np.frombuffer(json.dumps(dict(keys=list(sd), torch=torch.__version__, reference_commit="892eb57",
+                                                generator="oracle/make_golden.py default_init")).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(GOLDEN, "tiny_default_init.npz"), **out)
+    print("tiny_default_init  logits[0]=%s  %d state-dict entries" % (logits[0].tolist(), len(sd)))
+
+
+def data_pipeline_case():
+    """The reference's host-side input pipeline (code/utils_rd.py) on the raw arrays of
+    tests/test_data_pipeline.py::_raw(seed=4).  getStats is stored only where the installed numpy still accepts it
+    (numpy >= 1.24 rejects its `np.max([array, scalar])`); the rest runs on the restatement's statistics."""
+    from oracle import data_oracle as DO
+    from test_data_pipeline import _raw
+    ref_harness.load_reference()
+    import utils_rd as U
+    P, minutes, static, y = _raw(seed=4)
+    out = {}
+    mf, stdf = DO.get_stats(P)
+    try:
+        out["getStats.mf"], out["getStats.stdf"] = U.getStats(P)
+    except ValueError:
+        pass
+    out["mask_normalize"] = U.mask_normalize(P.copy(), mf, stdf)
+    ms, ss = U.getStats_static(static, dataset="P12")
+    out["getStats_static.ms"], out["getStats_static.ss"] = ms, ss
+    out["mask_normalize_static"] = U.mask_normalize_static(static.copy(), ms, ss)
+    Plist = [{"arr": P[i], "time": minutes[i][:, None], "extended_static": static[i]} for i in range(len(P))]
+    for i, t in enumerate(U.tensorize_normalize(Plist, y, mf, stdf, ms, ss)):
+        out["tensorize_normalize.%d" % i] = t.numpy()
+    np.savez_compressed(os.path.join(GOLDEN, "data_pipeline.npz"), **out)
+    print("data_pipeline      %d arrays: %s" % (len(out), sorted(out)))
 
 
 if __name__ == "__main__":
@@ -241,8 +300,16 @@ if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "v1":
         v1_case()
         sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "default_init":
+        default_init_case()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "data_pipeline":
+        data_pipeline_case()
+        sys.exit(0)
     for case in CASES:
         run_case(*case)
     operator_cases()
     operator_grad_cases()
     v1_case()
+    default_init_case()
+    data_pipeline_case()

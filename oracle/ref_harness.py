@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path (raindrop_b200/).
 
-Loads the reference's OWN, UNMODIFIED files (`/root/reference/code/{models_rd,Ob_propagation,
-transformer_conv}.py`) on CPU so they can be used (a) to pin the oracle restatement in
-`oracle/raindrop_oracle.py` and (b) to generate the committed golden fixtures under
-`tests/golden/` (script: `oracle/make_golden.py`).  `/root/reference` only exists in the
-build container; nothing that runs on the GPU box may call `load_reference()`.
+Loads the reference's OWN, UNMODIFIED files (`code/{models_rd,Ob_propagation,transformer_conv}.py`
+of a checkout of the original Raindrop project, located by the environment variable
+RAINDROP_REFERENCE) on CPU, to generate the committed golden fixtures under `tests/golden/`
+(script: `oracle/make_golden.py`) that pin the oracle restatement in `oracle/raindrop_oracle.py`
+and the CUDA path.  The tests read only those fixtures, never the reference itself.
 
 Why patches are needed (SURVEY.md section 8c):
   * torch_geometric / torch_scatter / torch_sparse are not installed -> `oracle/pyg_shim`.
@@ -22,7 +22,7 @@ import sys
 import torch
 import torch.nn as nn
 
-REFERENCE_CODE = "/root/reference/code"
+REFERENCE_CODE = os.path.join(os.path.abspath(os.environ.get("RAINDROP_REFERENCE") or os.devnull), "code")
 _SHIM = os.path.join(os.path.dirname(os.path.abspath(__file__)), "pyg_shim")
 _loaded = None
 
@@ -37,7 +37,7 @@ def load_reference():
     if _loaded is not None:
         return _loaded
     if not reference_available():
-        raise RuntimeError("reference tree not present (only exists in the build container)")
+        raise RuntimeError("reference tree not found: set RAINDROP_REFERENCE to a checkout of the original project")
     if torch.cuda.is_available():
         raise RuntimeError("the reference harness is CPU-only (it patches Tensor.cuda)")
 

@@ -115,23 +115,25 @@ def used_param_keys(cfg):
     return keys
 
 
+def keyed_values(seed, key, shape, scale=1.0):
+    """Values of state-dict entry `key` from the keyed stream: fan-in scaled uniform for matrices, LayerNorm
+    weights near one, other vectors near zero (perturbed so that every term is exercised)."""
+    u = torch.from_numpy(_stream(seed, key, int(np.prod(shape)))).view(shape).float()
+    if key.endswith("norm1.weight") or key.endswith("norm2.weight"):
+        return 1.0 + 0.2 * (u - 0.5)
+    if len(shape) == 1:
+        return 0.2 * (u - 0.5)
+    return (2 * u - 1) * (scale * (3.0 / shape[1]) ** 0.5)
+
+
 def synth_weights(model, cfg, seed=7, scale=1.0):
     """Overwrites the USED parameters of `model` (reference, oracle or drop-in: same keys) and its
-    `R_u` attribute with values from the keyed stream.  Fan-in scaled uniform, biases and LayerNorm
-    affine terms perturbed so that every term is exercised.  Returns R_u."""
+    `R_u` attribute with values from the keyed stream (`keyed_values`).  Returns R_u."""
     sd = model.state_dict()
     with torch.no_grad():
         for key in used_param_keys(cfg):
             t = sd[key]
-            u = torch.from_numpy(_stream(seed, key, t.numel())).view(t.shape).float()
-            if key.endswith("norm1.weight") or key.endswith("norm2.weight"):
-                val = 1.0 + 0.2 * (u - 0.5)
-            elif t.dim() == 1:
-                val = 0.2 * (u - 0.5)
-            else:
-                bound = scale * (3.0 / t.shape[1]) ** 0.5
-                val = (2 * u - 1) * bound
-            t.copy_(val)
+            t.copy_(keyed_values(seed, key, tuple(t.shape), scale))
         Dm = cfg["d_inp"] * cfg["d_ob"]
         r = torch.from_numpy(_stream(seed, "R_u", Dm)).float().view(1, Dm)
         r_u = (2 * r - 1) * 1.2

@@ -1,7 +1,6 @@
 """Input pipeline (raindrop_b200/data.py) against the CPU restatement of the reference's host code
 (oracle/data_oracle.py) -- and that restatement against the reference's own functions where they are present."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -10,8 +9,6 @@ import torch
 from helpers import normwise
 from oracle import data_oracle as DO
 from raindrop_b200 import data as RD
-
-REF = "/root/reference/code"
 
 
 def _raw(n=23, T=17, F=6, D=4, seed=0):
@@ -71,32 +68,27 @@ def test_removal_indices_match_reference_choice():
     assert list(RD.removal_indices(7, 34, 0.3, "set", density_scores=np.arange(34)[::-1])) == list(range(33, 23, -1))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_data_oracle_matches_reference():
-    """Pins oracle/data_oracle.py to the reference's own utils_rd functions (bit-identical float64 results)."""
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-    import ref_harness  # noqa: F401  (installs the shims the reference's imports need)
-    sys.path.insert(0, REF)
-    import utils_rd as U
+def test_data_oracle_matches_reference(golden_dir):
+    """Pins oracle/data_oracle.py to the reference's own utils_rd functions (bit-identical float64 results), stored by
+    oracle/make_golden.py data_pipeline_case for these raw arrays."""
+    z = np.load(os.path.join(golden_dir, "data_pipeline.npz"))
     P, minutes, static, y = _raw(seed=4)
-    mf2, stdf2 = DO.get_stats(P)
-    try:
-        mf, stdf = U.getStats(P)
-        assert np.array_equal(mf, mf2) and np.array_equal(stdf, stdf2)
-    except ValueError:
-        # numpy >= 1.24 rejects the reference's `np.max([stdf[f], eps])` (a (1,) array next to a scalar, code/utils_rd.py:160);
-        # the restatement is the same arithmetic on the scalar.  Check it against a direct computation instead.
-        Pf = P.transpose((2, 0, 1)).reshape(P.shape[2], -1)
-        for f in range(P.shape[2]):
-            v = Pf[f][Pf[f] > 0]
-            assert mf2[f, 0] == np.mean(v) and stdf2[f, 0] == max(np.std(v), 1e-7)
-        mf, stdf = mf2, stdf2
-    assert np.array_equal(U.mask_normalize(P.copy(), mf, stdf), DO.mask_normalize(P.copy(), mf, stdf))
-    ms, ss = U.getStats_static(static, dataset="P12")
+    mf, stdf = DO.get_stats(P)
+    if "getStats.mf" in z.files:
+        assert np.array_equal(z["getStats.mf"], mf) and np.array_equal(z["getStats.stdf"], stdf)
+    # numpy >= 1.24 rejects the reference's `np.max([stdf[f], eps])` (a (1,) array next to a scalar, code/utils_rd.py:160),
+    # so the fixture may lack getStats; the restatement is the same arithmetic on the scalar.  Check it against a direct
+    # computation as well.
+    Pf = P.transpose((2, 0, 1)).reshape(P.shape[2], -1)
+    for f in range(P.shape[2]):
+        v = Pf[f][Pf[f] > 0]
+        assert mf[f, 0] == np.mean(v) and stdf[f, 0] == max(np.std(v), 1e-7)
+    assert np.array_equal(z["mask_normalize"], DO.mask_normalize(P.copy(), mf, stdf))
+    ms, ss = z["getStats_static.ms"], z["getStats_static.ss"]
+    assert ms.shape == ss.shape == (static.shape[1], 1)
     assert (ms == 0).all() and (ss == 1).all()                           # the always-false categorical test
-    assert np.array_equal(U.mask_normalize_static(static.copy(), ms, ss), DO.mask_normalize_static(static))
-    Plist = [{"arr": P[i], "time": minutes[i][:, None], "extended_static": static[i]} for i in range(len(P))]
-    a = U.tensorize_normalize(Plist, y, mf, stdf, ms, ss)
+    assert np.array_equal(z["mask_normalize_static"], DO.mask_normalize_static(static))
+    a = [torch.from_numpy(z["tensorize_normalize.%d" % i]) for i in range(4)]
     b = DO.tensorize_normalize(P, minutes, static, y, mf, stdf)
     assert torch.equal(a[0].permute(1, 0, 2), b[0]) and torch.equal(a[1], b[1])
     assert torch.equal(a[2].squeeze(2).permute(1, 0), b[2]) and torch.equal(a[3], b[3])

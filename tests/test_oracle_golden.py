@@ -1,11 +1,13 @@
 """CPU: pins the oracle restatement (oracle/raindrop_oracle.py) against the golden fixtures that were
 generated from the reference's own unmodified files (oracle/make_golden.py)."""
+import json
+
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import case_setup, check_against_golden, load_golden, normwise
+from helpers import case_setup, check_against_golden, fingerprint, load_golden, normwise
 from oracle.raindrop_oracle import (ObPropOracle, TransformerConvOracle, build_oracle_model, encoder_layer_explicit,
                                     graph_from_adjacency, node_scale_from_graph, positional_encoding)
 from raindrop_b200.synth import synth_weights, used_param_keys
@@ -91,21 +93,27 @@ def test_graph_and_pe_conventions():
     assert abs(pe[0, 1, 7].item() - np.sin(np.float32(3.0) / np.float32(60.0))) < 1e-7
 
 
-def test_live_reference_if_present():
-    """In the build container the reference tree exists: run it directly against the oracle."""
-    from oracle import ref_harness
-    if not ref_harness.reference_available() or torch.cuda.is_available():
-        pytest.skip("reference tree only exists in the (GPU-less) build container")
+def test_oracle_matches_reference_default_init(golden_dir):
+    """Seeded construction (the modules' own initialisation, code/Raindrop.py:245-251) and the eval forward on it
+    against the reference's own model (oracle/make_golden.py default_init_case)."""
     from raindrop_b200.synth import make_batch, model_config
+    z = np.load(golden_dir + "/tiny_default_init.npz")
     cfg = model_config("TINY", dropout=0.2)
-    ref = ref_harness.build_reference_model(cfg).eval()
     orc = build_oracle_model(cfg).eval()
-    assert all(torch.equal(a, b) for a, b in zip(ref.state_dict().values(), orc.state_dict().values()))
+    sd = orc.state_dict()
+    assert list(sd) == json.loads(bytes(z["meta"]).decode())["keys"]
+    for k, v in sd.items():
+        if "sd." + k in z.files:
+            assert np.array_equal(v.numpy(), z["sd." + k]), k
+        else:
+            fp = fingerprint(v)
+            assert np.array_equal(fp["sample"], z["sd." + k + "#sample"]), k
+            assert np.allclose(fp["stats"], z["sd." + k + "#stats"], rtol=1e-12, atol=0), k
     batch = make_batch(cfg, 3, seed=1)
     with torch.no_grad():
-        a = ref.forward(batch["src"], batch["static"], batch["times"], batch["lengths"])[0]
         b = orc.forward(batch["src"], batch["static"], batch["times"], batch["lengths"])[0]
-    assert torch.equal(a, b)
+    # stored on another machine: CPU GEMM kernels may round the last bit differently there
+    assert normwise(b, z["logits"]) < 1e-6
 
 
 @pytest.mark.parametrize("seed", range(6))
