@@ -211,6 +211,27 @@ int rd_raindrop_v2_bwd(const rd_dims* dims, const rd_params* params, const float
                        const float* d_logits, const rd_grads* grads, void* scratch, int32_t phases,
                        void* stream);
 
+/* Gradients with respect to the float inputs of Raindrop_v2.forward (code/models_rd.py:278-296, 33-35), written, not
+ * accumulated.  Any member may be NULL (not wanted).
+ *   src     [T, B, 2N]   value half through the lift relu(v * R_u) and its dropout; the mask half is exactly 0
+ *   statics [B, d_static] through emb (needs d_static > 0)
+ *   times   [T, B]       through the positional encoding                                                      */
+typedef struct rd_input_grads {
+  float* src;
+  float* statics;
+  float* times;
+} rd_input_grads;
+/* bytes of `in_scratch` for rd_raindrop_v2_bwd_inputs (W1^T with its remainder, or the fallback's d(lifted input)) */
+size_t rd_input_grad_scratch_bytes(const rd_dims* dims);
+/* The whole backward of rd_raindrop_v2_fwd with input gradients.  grads == NULL: no parameter gradient is computed
+ * (frozen model, attribution): the weight-gradient GEMMs, LayerNorm column sums and head parameter outputs are
+ * skipped.  grads != NULL: every parameter gradient is bit-identical to rd_raindrop_v2_bwd(..., RD_BWD_ALL).
+ * scratch: rd_backward_scratch_bytes(dims) bytes; in_scratch: rd_input_grad_scratch_bytes(dims) bytes. */
+int rd_raindrop_v2_bwd_inputs(const rd_dims* dims, const rd_params* params, const float* statics,
+                              const int64_t* lengths, const float* node_scale, const void* workspace,
+                              const float* d_logits, const rd_grads* grads, const rd_input_grads* in_grads,
+                              void* scratch, void* in_scratch, void* stream);
+
 /* ---- temporal encoder + pooling + head on a caller-provided encoder input ------------------------------------
  * The second half of Raindrop_v2.forward (code/models_rd.py:354-385) and all of legacy Raindrop v1 after its
  * per-sample TransformerConv (code/models_rd.py:168-191): nn.TransformerEncoder with key-padding mask, masked mean

@@ -297,6 +297,7 @@ int head_bwd(int B, int T, int D, int N, int ds, int ncls, const int64_t* length
   if (smem > 48 * 1024) { set_error("head_bwd: feature width %d too large", p.Df); return -2; }
   launch_pdl(head_bwd_sample_kernel, dim3(B), dim3(HT), smem, st, p, hpre, dlogits, dh, dfeat, dx);
   RD_CHECK_LAUNCH("head_bwd_sample_kernel");
+  if (!g_w0) return 0;      // input gradients only: dfeat and dx are all the caller needs
   OuterGroup g;
   g.B = B; g.n = 0;
   int blk = 0;

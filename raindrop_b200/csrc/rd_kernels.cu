@@ -261,6 +261,56 @@ __global__ void lift_posenc_kernel(const float* __restrict__ src, const float* _
   pe_out[tok * ld + col0 + j] = (j < half) ? sinf(scaled) : cosf(scaled);
 }
 
+// Input gradients that need no GEMM, in one launch (segments as in lift_posenc_kernel):
+//   o <  n_src            : token (t, b), sensor n: d_src[t, b, N + n] = 0 (the mask half takes no part in the output,
+//                           code/models_rd.py:290); with dX0 (CUDA-core fallback of the lift backward, already gated and
+//                           scaled) also d_src[t, b, n] = sum_k dX0[(b*N+n), t*d_ob+k] * R_u[n*d_ob+k]
+//   next n_times          : d_times[tok] = sum_j (dZ[tok, pe+j] Z[tok, pe+h+j] - dZ[tok, pe+h+j] Z[tok, pe+j]) / ts_j,
+//                           from the saved sin / cos columns of the encoder input (code/models_rd.py:33-35)
+//   next n_static         : d_static[b, i] = sum_j dfeat[b, D+j] emb_w[j, i]        (code/models_rd.py:293-294)
+__global__ void input_grad_tail_kernel(int B, int T, int N, int d_ob, int D, int pe_col, const float* __restrict__ dZ,
+                                       const float* __restrict__ Z, TS8 ts, const float* __restrict__ dfeat, int Df,
+                                       const float* __restrict__ emb_w, int ds, const float* __restrict__ dX0,
+                                       const float* __restrict__ R_u, long long n_src, long long n_times,
+                                       long long n_static, float* __restrict__ d_src, float* __restrict__ d_times,
+                                       float* __restrict__ d_static) {
+  pdl_launch_dependents();
+  pdl_wait();
+  long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (o < n_src) {
+    const long long tok = o / N;
+    const int n = (int)(o - tok * N);
+    float* dst = d_src + tok * (2LL * N);
+    dst[N + n] = 0.f;
+    if (dX0) {
+      const int t = (int)(tok / B), b = (int)(tok - (long long)t * B);
+      const float* g = dX0 + ((long long)b * N + n) * ((long long)T * d_ob) + (long long)t * d_ob;
+      float a = 0.f;
+      for (int k = 0; k < d_ob; ++k) a += g[k] * __ldg(R_u + n * d_ob + k);
+      dst[n] = a;
+    }
+    return;
+  }
+  o -= n_src;
+  if (o < n_times) {
+    const int h = ts.d_pe >> 1;
+    const float* dz = dZ + o * D + pe_col;
+    const float* z = Z + o * D + pe_col;
+    float a = 0.f;
+    for (int j = 0; j < h; ++j) a += (dz[j] * z[h + j] - dz[h + j] * z[j]) / ts.v[j];
+    d_times[o] = a;
+    return;
+  }
+  o -= n_times;
+  if (o < n_static) {
+    const int b = (int)(o / ds), i = (int)(o - (long long)b * ds);
+    const float* df = dfeat + (long long)b * Df + D;
+    float a = 0.f;
+    for (int j = 0; j < N; ++j) a += df[j] * __ldg(emb_w + (long long)j * ds + i);
+    d_static[o] = a;
+  }
+}
+
 // one warp per node: segment max, then sum of exp, then s = sum(exp / (sum + 1e-16))
 __global__ void node_scale_kernel(const int64_t* __restrict__ tgt, const float* __restrict__ w, int E, int N,
                                   float* __restrict__ s) {
@@ -838,6 +888,25 @@ int lift_posenc(const float* src, const float* R_u, int B, int T, int N, int d_o
 int posenc(const float* times, int64_t n_tokens, const float* ts_host, int d_pe, float* out, int64_t ld, int col0,
            cudaStream_t st) {
   return lift_posenc(nullptr, nullptr, 0, 0, 0, 0, 0.f, nullptr, 0, nullptr, times, n_tokens, ts_host, d_pe, out, ld, col0, st);
+}
+
+int input_grad_tail(int B, int T, int N, int d_ob, int D, const float* dZ, const float* Z, const float* ts_host,
+                    int d_pe, const float* dfeat, int Df, const float* emb_w, int ds, const float* dX0, const float* R_u,
+                    float* d_src, float* d_times, float* d_static, cudaStream_t st) {
+  if (d_pe < 2 || d_pe > 64 || (d_pe & 1)) { set_error("input_grad_tail: positional encoding width must be even and <= 64"); return -2; }
+  const int64_t n_src = d_src ? (int64_t)T * B * N : 0;
+  const int64_t n_times = d_times ? (int64_t)T * B : 0;
+  const int64_t n_static = d_static ? (int64_t)B * ds : 0;
+  TS8 ts;
+  memset(&ts, 0, sizeof(ts));
+  ts.d_pe = d_pe;
+  memcpy(ts.v, ts_host, sizeof(float) * (d_pe / 2));
+  const int64_t total = n_src + n_times + n_static;
+  if (total <= 0) return 0;
+  launch_pdl(input_grad_tail_kernel, dim3(blocks_for(total)), dim3(TPB), 0, st, B, T, N, d_ob, D, D - d_pe, dZ, Z, ts, dfeat,
+             Df, emb_w, ds, dX0, R_u, (long long)n_src, (long long)n_times, (long long)n_static, d_src, d_times, d_static);
+  RD_CHECK_LAUNCH("input_grad_tail_kernel");
+  return 0;
 }
 
 int node_scale(const int64_t* edge_tgt, const float* edge_w, int E, int N, float* s, cudaStream_t st) {

@@ -65,7 +65,7 @@ int head_fwd(int B, int T, int D, int N, int ds, int ncls, const float* x, const
              const float* emb_w, const float* emb_b, const float* w0, const float* b0, const float* w2, const float* b2,
              float* feat, float* hpre, float* logits, const int64_t* y, float* loss_ps, float* dlogits, float* loss,
              unsigned* counter, cudaStream_t st);
-// dx = d(loss)/d(encoder output) [T, B, D] (masked-mean backward)
+// dx = d(loss)/d(encoder output) [T, B, D] (masked-mean backward); g_w0 == null: no parameter gradients (no second launch)
 int head_bwd(int B, int T, int D, int N, int ds, int ncls, const int64_t* lengths, const float* statics, const float* w0,
              const float* w2, const float* feat, const float* hpre, const float* dlogits, float* dh, float* dfeat, float* dx,
              float* g_w0, float* g_b0, float* g_w2, float* g_b2, float* g_emb_w, float* g_emb_b, cudaStream_t st);
@@ -88,6 +88,15 @@ int attn_tc_bwd(const float* qkv, const float* dctx, const int64_t* lengths, int
 // dZ2[(b*N+n), t*d_ob+k] = dZ[t,b,n*d_ob+k] * s[n] * (Z[t,b,n*d_ob+k] > 0)
 int obprop_out_grad(const float* dZ, const float* Z, const float* s, int B, int T, int N, int d_ob, int D,
                     int round, float* dZ2, cudaStream_t st);
+
+// Input gradients of Raindrop_v2 that need no GEMM, one launch (each output may be null):
+//   d_src [T, B, 2N]: mask half zeroed; value half from dX0 [B*N, T*d_ob] (gated, scaled: the CUDA-core fallback of the
+//                     lift backward) when dX0 != null, else left to the tensor-core store
+//   d_times [T, B]  : from dZ / Z [T, B, D] (the encoder input's last d_pe columns are sin | cos of times / ts_host[j])
+//   d_static [B, ds]: dfeat[b, D : D+N] . emb_w [N, ds]   (dfeat [B, Df] from head_bwd)
+int input_grad_tail(int B, int T, int N, int d_ob, int D, const float* dZ, const float* Z, const float* ts_host,
+                    int d_pe, const float* dfeat, int Df, const float* emb_w, int ds, const float* dX0, const float* R_u,
+                    float* d_src, float* d_times, float* d_static, cudaStream_t st);
 
 // y[i] = x[i] * mask(site, i)   (re-generates the forward's dropout mask)
 int apply_dropout(const float* x, int64_t n, float p, const uint64_t* rng, uint32_t site, float* y,

@@ -114,6 +114,24 @@ struct BwLayout {
   int64_t partial_floats;
 };
 
+// Input-gradient scratch (rd_input_grad_scratch_bytes).  The lift backward dX0 = gO1 . W1 runs on the ob-prop tensor-core
+// kernel against W1^T and its remainder, derived in the backward (the forward cannot know whether input gradients will
+// be asked for); shapes that kernel does not take go through the CUDA-core GEMM into dX0.
+struct InLayout { int64_t W1t, W1tlo, dX0, total; };
+
+bool lift_bwd_tc(const Shape& s) { return s.tc && s.dob == 4; }
+
+InLayout in_layout(const Shape& s) {
+  InLayout l;
+  Arena a;
+  const int64_t cc = lift_bwd_tc(s) ? (int64_t)s.C * s.C : 0;
+  l.W1t = a.take(cc);
+  l.W1tlo = a.take(cc);
+  l.dX0 = a.take(lift_bwd_tc(s) ? 0 : s.M1 * s.C);
+  l.total = a.off;
+  return l;
+}
+
 int64_t splitk_partial_floats(int Nout, int Kin, int64_t rows) {
   int ns;
   return gemm_splitk_plan(Nout, Kin, (int)rows, &ns);
@@ -385,12 +403,19 @@ static int raindrop_fwd(const rd_dims* dims, const rd_params* P, const float* sr
 
 static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* statics, const int64_t* lengths,
                         const float* nscale, const float* ws, const float* dlogits, const rd_grads* G, float* sc,
-                        int phases, float* d_z0_out, cudaStream_t st) {
+                        int phases, float* d_z0_out, cudaStream_t st, const rd_input_grads* IG = nullptr,
+                        float* isc = nullptr) {
   Shape s;
   RD_TRY(make_shape(dims, &s));
   if ((phases & ~3) || phases == 0) { set_error("rd_raindrop_v2_bwd: phases must be 1, 2 or 3"); return -2; }
   WsLayout w = ws_layout(s);
   BwLayout b = bw_layout(s);
+  // G == null: input gradients only.  Every weight-gradient enqueue (tn), LayerNorm column sum and the head's parameter
+  // outputs are skipped; the input-gradient chain itself is the same launches as with parameter gradients.
+  const bool pg = G != nullptr;
+  const rd_grads none = {};
+  if (!pg) G = &none;
+  const bool d_src = IG && IG->src;
   const uint64_t* rng = reinterpret_cast<const uint64_t*>(ws + w.rng);
   float* partial = sc + b.partial;
   const float ik = s.p > 0.f ? 1.f / (1.f - s.p) : 1.f;
@@ -433,15 +458,17 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
     }
     RD_TRY(layernorm_bwd(r2, ws + w.l[l].st2, E.norm2_weight, gA, s.M2, s.D, res, GE.norm2_weight, GE.norm2_bias,
                          sc + b.l[l].ln[0], K2, s.p, rng, SITE_RESID2 + l, &chunks, st, m2, mld));
-    RD_TRY(wq.colsum(sc + b.l[l].ln[0], 2 * s.D, chunks, s.D, GE.norm2_weight, st));
-    RD_TRY(wq.colsum(sc + b.l[l].ln[0] + s.D, 2 * s.D, chunks, s.D, GE.norm2_bias, st));
-    RD_TRY(tn(&wq, K2, s.D, f, s.nhid, GE.linear2_weight, GE.linear2_bias, s.D, s.nhid, s.M2, sc + b.l[l].wp[0], partial, st));
+    if (pg) {
+      RD_TRY(wq.colsum(sc + b.l[l].ln[0], 2 * s.D, chunks, s.D, GE.norm2_weight, st));
+      RD_TRY(wq.colsum(sc + b.l[l].ln[0] + s.D, 2 * s.D, chunks, s.D, GE.norm2_bias, st));
+      RD_TRY(tn(&wq, K2, s.D, f, s.nhid, GE.linear2_weight, GE.linear2_bias, s.D, s.nhid, s.M2, sc + b.l[l].wp[0], partial, st));
+    }
     {   // gF = (K2 . W2) * [f > 0] / (1-p)   ("NT" against W2^T so that the tensor-core kernel applies)
       GemmP g = nt(K2, s.D, ws + w.wsp[l].l2_t, s.D, gF, s.nhid, s.M2, s.nhid, s.D);
       g.gate = f; g.gate_ld = s.nhid; g.gate_scale = ik;  // relu' and the FFN dropout mask in one
       RD_TRY(linear_nt(g, ws + w.wsp[l].l2_tlo, st));
     }
-    RD_TRY(tn(&wq, gF, s.nhid, x1, s.D, GE.linear1_weight, GE.linear1_bias, s.nhid, s.D, s.M2, sc + b.l[l].wp[1], partial, st));
+    if (pg) RD_TRY(tn(&wq, gF, s.nhid, x1, s.D, GE.linear1_weight, GE.linear1_bias, s.nhid, s.D, s.M2, sc + b.l[l].wp[1], partial, st));
     {
       GemmP g = nt(gF, s.nhid, ws + w.wsp[l].l1_t, s.nhid, gA, s.D, s.M2, s.D, s.nhid);
       g.resid = res; g.resid_ld = s.D;
@@ -451,9 +478,11 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
     res = s.p > 0.f ? gB : K1;
     RD_TRY(layernorm_bwd(r1, ws + w.l[l].st1, E.norm1_weight, gA, s.M2, s.D, res, GE.norm1_weight, GE.norm1_bias,
                          sc + b.l[l].ln[1], K1, s.p, rng, SITE_RESID1 + l, &chunks, st, m1, mld));
-    RD_TRY(wq.colsum(sc + b.l[l].ln[1], 2 * s.D, chunks, s.D, GE.norm1_weight, st));
-    RD_TRY(wq.colsum(sc + b.l[l].ln[1] + s.D, 2 * s.D, chunks, s.D, GE.norm1_bias, st));
-    RD_TRY(tn(&wq, K1, s.D, ctx, s.D, GE.out_proj_weight, GE.out_proj_bias, s.D, s.D, s.M2, sc + b.l[l].wp[2], partial, st));
+    if (pg) {
+      RD_TRY(wq.colsum(sc + b.l[l].ln[1], 2 * s.D, chunks, s.D, GE.norm1_weight, st));
+      RD_TRY(wq.colsum(sc + b.l[l].ln[1] + s.D, 2 * s.D, chunks, s.D, GE.norm1_bias, st));
+      RD_TRY(tn(&wq, K1, s.D, ctx, s.D, GE.out_proj_weight, GE.out_proj_bias, s.D, s.D, s.M2, sc + b.l[l].wp[2], partial, st));
+    }
     RD_TRY(linear_nt(nt(K1, s.D, ws + w.wsp[l].out_t, s.D, gD, s.D, s.M2, s.D, s.D), ws + w.wsp[l].out_tlo, st));
     if (attn_tc_supported(s.T, s.hd)) {
       RD_TRY(attn_tc_bwd(qkv, gD, lengths, s.B, s.H, s.T, s.hd, s.p, rng, SITE_ATTN + l, dqkv, st));
@@ -494,7 +523,7 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
         RD_TRY(gemm(g, st));
       }
     }
-    RD_TRY(tn(&wq, dqkv, 3 * s.D, x, s.D, GE.in_proj_weight, GE.in_proj_bias, 3 * s.D, s.D, s.M2, sc + b.l[l].wp[3], partial, st));
+    if (pg) RD_TRY(tn(&wq, dqkv, 3 * s.D, x, s.D, GE.in_proj_weight, GE.in_proj_bias, 3 * s.D, s.D, s.M2, sc + b.l[l].wp[3], partial, st));
     {
       // the first layer's input gradient is d(loss)/d(encoder input): optionally delivered straight to the caller
       GemmP g = nt(dqkv, 3 * s.D, ws + w.wsp[l].in_t, 3 * s.D, (l == 0 && d_z0_out) ? d_z0_out : gA, s.D, s.M2, s.D, 3 * s.D);
@@ -505,13 +534,14 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
   if (!(phases & RD_BWD_OBPROP)) RD_TRY(wq.flush(st));   // encoder + head gradients complete: the caller may reduce them now
   }
 
-  if (phases & RD_BWD_OBPROP) {
+  // with neither parameter gradients nor d_src wanted nothing below the encoder input is needed
+  if ((phases & RD_BWD_OBPROP) && (pg || d_src)) {
   // ---- observation propagation: gA = d(loss)/d(Z0) [T,B,D]          code/models_rd.py:322-343
   float* gO2 = sc + b.gO2; float* gO1 = sc + b.gO1;
   const float* X0 = ws + w.X0; const float* H1 = ws + w.H1;
   const int tc = s.tc;
   RD_TRY(obprop_out_grad(gA, ws + w.Z[0], nscale, s.B, s.T, s.N, s.dob, s.D, tc && !s.exact, gO2, st));
-  RD_TRY(tn(&wq, gO2, s.C, H1, s.C, G->ob2_value_weight, G->ob2_value_bias, s.C, s.C, s.M1, sc + b.wp_ob[0], partial, st));
+  if (pg) RD_TRY(tn(&wq, gO2, s.C, H1, s.C, G->ob2_value_weight, G->ob2_value_bias, s.C, s.C, s.M1, sc + b.wp_ob[0], partial, st));
   if (tc) {
     // dZ1 = (dZ2 . W2) * s * [H1 > 0] on the tensor cores: "NT" form against a transposed, TF32-rounded W2
     const float* W2t = ws + w.W2t;      // written by the forward's weight-prep launch
@@ -525,8 +555,34 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
     g.rowscale = nscale; g.rowscale_mod = s.N; g.gate = H1; g.gate_ld = s.C;
     RD_TRY(gemm(g, st));
   }
-  RD_TRY(tn(&wq, gO1, s.C, X0, s.C, G->ob1_value_weight, G->ob1_value_bias, s.C, s.C, s.M1, sc + b.wp_ob[1], partial, st));
+  if (pg) RD_TRY(tn(&wq, gO1, s.C, X0, s.C, G->ob1_value_weight, G->ob1_value_bias, s.C, s.C, s.M1, sc + b.wp_ob[1], partial, st));
   RD_TRY(wq.flush(st));
+  if (d_src) {
+    // dX0 = gO1 . W1, gated by X0 != 0 (relu' of the lift and its dropout keep bit at once: X0 is non-zero exactly where
+    // both are 1) and scaled by 1/(1-p), then reduced over the d_ob channels against R_u.  Always error-compensated:
+    // gO1 is not TF32-rounded (rounding it would change the ob1 weight gradient)
+    const float ik = s.p > 0.f ? 1.f / (1.f - s.p) : 1.f;
+    const InLayout il = in_layout(s);
+    if (lift_bwd_tc(s)) {
+      WeightSplit it = {P->ob1_value_weight, s.C, s.C, nullptr, isc + il.W1t, isc + il.W1tlo};
+      RD_TRY(split_weights(&it, 1, st));
+      ObpropTcArgs a;
+      a.x = gO1; a.W = isc + il.W1t; a.W_lo = isc + il.W1tlo; a.bias = nullptr; a.relu = 0; a.gate = X0;
+      a.rows = s.M1; a.C = s.C; a.out = IG->src;
+      a.pB = s.B; a.pN = s.N; a.pdob = s.dob; a.pD = 2 * s.N;
+      a.lift_ru = P->R_u; a.lift_scale = ik;
+      RD_TRY(obprop_tc_fwd(a, st));
+    } else {
+      GemmP g = nn(gO1, s.C, P->ob1_value_weight, s.C, isc + il.dX0, s.C, s.M1, s.C, s.C);
+      g.gate = X0; g.gate_ld = s.C; g.gate_scale = ik;
+      RD_TRY(gemm(g, st));
+    }
+  }
+  }
+  if (IG && (IG->src || IG->times || IG->statics)) {
+    RD_TRY(input_grad_tail(s.B, s.T, s.N, s.dob, s.D, gA, ws + w.Z[0], dims->pe_timescales, RD_D_PE, sc + b.dfeat, s.Df,
+                           P->emb_weight, s.ds, (d_src && !lift_bwd_tc(s)) ? isc + in_layout(s).dX0 : nullptr, P->R_u,
+                           IG->src, IG->times, IG->statics, st));
   }
   return 0;
 }
@@ -724,6 +780,30 @@ int rd_raindrop_v2_bwd(const rd_dims* dims, const rd_params* params, const float
   }
   return raindrop_bwd(dims, params, statics, lengths, node_scale, (const float*)workspace, d_logits, grads,
                       (float*)scratch, phases, nullptr, (cudaStream_t)stream);
+}
+
+size_t rd_input_grad_scratch_bytes(const rd_dims* dims) {
+  Shape s;
+  if (make_shape(dims, &s) != 0) return 0;
+  return (size_t)in_layout(s).total * sizeof(float);
+}
+
+int rd_raindrop_v2_bwd_inputs(const rd_dims* dims, const rd_params* params, const float* statics, const int64_t* lengths,
+                              const float* node_scale, const void* workspace, const float* d_logits, const rd_grads* grads,
+                              const rd_input_grads* in_grads, void* scratch, void* in_scratch, void* stream) {
+  if (!dims || !params || !lengths || !node_scale || !workspace || !d_logits || !scratch) {
+    set_error("rd_raindrop_v2_bwd_inputs: NULL argument");
+    return -2;
+  }
+  const bool any_in = in_grads && (in_grads->src || in_grads->statics || in_grads->times);
+  if (!grads && !any_in) { set_error("rd_raindrop_v2_bwd_inputs: neither parameter nor input gradients requested"); return -2; }
+  if (any_in && in_grads->src && !in_scratch) { set_error("rd_raindrop_v2_bwd_inputs: d_src needs in_scratch"); return -2; }
+  if (any_in && in_grads->statics && (dims->d_static < 1 || !statics)) {
+    set_error("rd_raindrop_v2_bwd_inputs: a static gradient needs d_static > 0 and statics");
+    return -2;
+  }
+  return raindrop_bwd(dims, params, statics, lengths, node_scale, (const float*)workspace, d_logits, grads, (float*)scratch,
+                      RD_BWD_ALL, nullptr, (cudaStream_t)stream, any_in ? in_grads : nullptr, (float*)in_scratch);
 }
 
 int rd_positional_encoding(const float* times, int64_t n_tokens, const float* timescales_host, int32_t d_pe, float* out,

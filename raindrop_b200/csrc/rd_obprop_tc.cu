@@ -48,6 +48,8 @@ struct TcParams {
   int relu, round_out;
   int perm, pB, pN, pD;
   float* out;
+  const float* lift_ru;
+  float lift_scale;
 };
 
 __device__ __forceinline__ float epi1(float acc, float bias, float sc, int relu, int rnd) {
@@ -61,7 +63,10 @@ __device__ __forceinline__ float epi1(float acc, float bias, float sc, int relu,
 // EXACT: error-compensated products (3xTF32, fp32-level accuracy) for the latency-bound row counts where the
 // tensor pipe has slack: the weight tile comes with its precomputed remainder (tmWlo), four extra warps derive the
 // activation remainder x - trunc19(x) in shared memory, and every k-step issues lo.hi + hi.lo + hi.hi.
-template <bool PERM, bool GATE, bool RELU, bool ROUND, bool EXACT>
+// LIFT_BWD: the input-gradient store of the lift X0 = dropout(relu(v * R_u)): a lane's 4 columns of one timestamp are
+// gated by X0 != 0 (relu' and the keep bit at once), weighted by R_u and summed into ONE value of d_src [T, B, 2N];
+// consecutive lanes are consecutive sensors, so the warp's stores coalesce.
+template <bool PERM, bool GATE, bool RELU, bool ROUND, bool EXACT, bool LIFT_BWD = false>
 __global__ void __launch_bounds__(EXACT ? NTHREADS_EXACT : NTHREADS, 1)
 obprop_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                  const __grid_constant__ CUtensorMap tmWlo, const __grid_constant__ CUtensorMap tmOut, const TcParams p) {
@@ -189,9 +194,16 @@ obprop_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       asm volatile("bar.sync 1, 128;" ::: "memory");
       const int row0 = m_t * BM + q * 32;
       const int row = row0 + lane;
-      const float sc = row < p.M ? __ldg(p.scale + (row % p.scale_mod)) : 0.f;
+      const float sc = (!LIFT_BWD && row < p.M) ? __ldg(p.scale + (row % p.scale_mod)) : 0.f;
       mbar_wait(tfull_bar(acc), acc_phase);
       tc_fence_after();
+      float* lift_row = nullptr;
+      float4 ru = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (LIFT_BWD && row < p.M) {
+        const int b = row / p.pN, n = row - b * p.pN;
+        lift_row = p.out + (size_t)b * p.pD + n;
+        ru = __ldg(reinterpret_cast<const float4*>(p.lift_ru) + n);
+      }
       // perm: this lane's row is sensor n of sample b; its 4 values of one timestamp are 16
       // contiguous bytes of out[t, b, n*4 .. n*4+3] and consecutive lanes are consecutive sensors,
       // so one st.global.v4 per timestamp is a fully coalesced 512-byte warp store (no staging).
@@ -205,6 +217,23 @@ obprop_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * 256 + ch * 32), v);
         const float* bs = bias_s + acc * 256 + ch * 32;
         const int c0 = col0 + ch * 32;
+        if (LIFT_BWD) {
+          if (lift_row) {
+#pragma unroll
+            for (int j4 = 0; j4 < 8; ++j4) {
+              const int t = (c0 >> 2) + j4;
+              if (4 * t < p.C && ch * 32 + 4 * j4 < p.BN) {
+                const float4 g = __ldg(reinterpret_cast<const float4*>(p.gate + (size_t)row * p.C + 4 * t));
+                float s = g.x != 0.f ? __uint_as_float(v[4 * j4 + 0]) * ru.x : 0.f;
+                s += g.y != 0.f ? __uint_as_float(v[4 * j4 + 1]) * ru.y : 0.f;
+                s += g.z != 0.f ? __uint_as_float(v[4 * j4 + 2]) * ru.z : 0.f;
+                s += g.w != 0.f ? __uint_as_float(v[4 * j4 + 3]) * ru.w : 0.f;
+                lift_row[(size_t)t * p.pB * p.pD] = s * p.lift_scale;
+              }
+            }
+          }
+          continue;
+        }
         if (PERM) {
           if (perm_row) {
 #pragma unroll
@@ -314,6 +343,13 @@ int obprop_tc_fwd(const ObpropTcArgs& a, cudaStream_t st) {
   const int64_t rows = a.rows; const int C = a.C; const int perm = a.perm, pB = a.pB, pN = a.pN, pdob = a.pdob, pD = a.pD;
   if (perm && pdob != 4) { set_error("obprop_tc_fwd: permuted store needs d_ob == 4"); return -2; }
   if (perm && a.gate) { set_error("obprop_tc_fwd: gate is only built for the plain layout"); return -2; }
+  const bool lift = a.lift_ru != nullptr;
+  if (lift && (perm || !a.gate || !a.W_lo || a.bias || a.relu || a.round_out || pdob != 4 ||
+               (reinterpret_cast<uintptr_t>(a.lift_ru) & 15))) {
+    set_error("obprop_tc_fwd: the lift-backward store needs d_ob == 4, the X0 gate, the error-compensated mode, no "
+              "bias / relu / rounding and a 16-byte aligned R_u");
+    return -2;
+  }
   if (rows > 0x7fffffffLL) { set_error("obprop_tc_fwd: too many rows"); return -2; }
   if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(out) |
        reinterpret_cast<uintptr_t>(a.gate)) & 15) {
@@ -336,6 +372,7 @@ int obprop_tc_fwd(const ObpropTcArgs& a, cudaStream_t st) {
   p.bias = a.bias; p.scale = a.scale; p.scale_mod = a.scale_mod; p.gate = a.gate;
   p.relu = a.relu; p.round_out = a.round_out;
   p.perm = perm; p.pB = pB; p.pN = pN; p.pD = pD; p.out = out;
+  p.lift_ru = a.lift_ru; p.lift_scale = a.lift_scale;
 
   CUtensorMap tmA, tmW, tmWlo, tmOut;
   {
@@ -352,13 +389,13 @@ int obprop_tc_fwd(const ObpropTcArgs& a, cudaStream_t st) {
     if (exact) RD_TRY(encode(&tmWlo, a.W_lo, 2, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, "W_lo"));
     else tmWlo = tmW;
   }
-  if (!perm) {
+  if (!perm && !lift) {
     cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
     cuuint64_t str[1] = {(cuuint64_t)C * 4};
     cuuint32_t box[2] = {32, 32};
     RD_TRY(encode(&tmOut, out, 2, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B, "out"));
   } else {
-    tmOut = tmA;   // permuted output is written with plain vector stores; the map is not used
+    tmOut = tmA;   // permuted / lift-backward output is written with plain stores; the map is not used
   }
   int total = p.m_tiles * p.n_tiles;
   int grid = total < num_sms() ? total : num_sms();
@@ -377,7 +414,8 @@ int obprop_tc_fwd(const ObpropTcArgs& a, cudaStream_t st) {
     else { set_error("obprop_tc_fwd: epilogue combination not instantiated"); return -2; }
   } else {
     if (rnd) { set_error("obprop_tc_fwd: the error-compensated mode does not round its output"); return -2; }
-    if (perm && !a.gate && relu) rc = launch(obprop_tc_kernel<true, false, true, false, true>, NTHREADS_EXACT);
+    if (lift) rc = launch(obprop_tc_kernel<false, true, false, false, true, true>, NTHREADS_EXACT);         // backward d(src)
+    else if (perm && !a.gate && relu) rc = launch(obprop_tc_kernel<true, false, true, false, true>, NTHREADS_EXACT);
     else if (!perm && !a.gate && relu) rc = launch(obprop_tc_kernel<false, false, true, false, true>, NTHREADS_EXACT);
     else if (!perm && a.gate && !relu) rc = launch(obprop_tc_kernel<false, true, false, false, true>, NTHREADS_EXACT);
     else { set_error("obprop_tc_fwd: epilogue combination not instantiated"); return -2; }

@@ -24,6 +24,10 @@ struct ObpropTcArgs {
   int relu = 1, round_out = 0;
   int64_t rows = 0; int C = 0; float* out = nullptr;
   int perm = 0, pB = 0, pN = 0, pdob = 0, pD = 0;
+  // lift_ru != null: backward of the input lift X0 = dropout(relu(v * R_u)) (needs d_ob == 4, gate = X0, W_lo, no
+  // bias / relu / scale): row r = b*pN + n, col c = t*4 + k  ->
+  //   out[(t*pB + b)*pD + n] = lift_scale * sum_k acc[r, 4t+k] * R_u[4n+k] * [gate[r, 4t+k] != 0]
+  const float* lift_ru = nullptr; float lift_scale = 1.f;
 };
 int obprop_tc_fwd(const ObpropTcArgs& a, cudaStream_t st);
 // Which mode a [rows, C] layer should run in (mode: 0 automatic, 1 single-pass TF32, 2 error-compensated).  Automatic =

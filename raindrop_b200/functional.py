@@ -153,6 +153,7 @@ class RaindropV2Function(torch.autograd.Function):
         ctx.plan, ctx.dims, ctx.P, ctx.ws, ctx.pool = plan, dims, P, ws, pool
         ctx.keep = (keep, static, lengths, plan.node_scale, plan.R_u)
         ctx.sc_bytes = sc_bytes
+        ctx.src_shape = tuple(src.shape)
         if plan.debug_keep_workspace:      # parity tests read named activation buffers (workspace_view)
             plan.last_workspace = ws
             plan.last_dims = dims
@@ -172,30 +173,14 @@ class RaindropV2Function(torch.autograd.Function):
         d_logits = _as_f32(d_logits)
         dev = d_logits.device
         params = keep
-        layout = plan.__dict__.get("_grad_layout")
-        if layout is None:      # tightly packed flat bucket, one offset per used parameter
-            offs, total = [], 0
-            for t in params:
-                offs.append(total)
-                total += t.numel()
-            layout = plan.__dict__["_grad_layout"] = (offs, total)
-        offs, total = layout
+        need = ctx.needs_input_grad
+        want_in = (need[2], need[3] and static is not None, need[4])      # src, static, times
+        want_params = any(need[6:])
+        if any(want_in) or not want_params:
+            return _backward_with_inputs(ctx, d_logits, want_in, want_params)
         owner = plan.owner() if plan.owner is not None else None
-        flat = torch.empty(total, dtype=torch.float32, device=dev)
-        base = flat.data_ptr()
-        cachedG = plan.__dict__.get("_grad_struct")
-        if cachedG is not None and cachedG[0] == base:
-            G = cachedG[1]
-        else:
-            G = L.RdGrads()
-            for (key, path), off in zip(plan.fields, offs):
-                _set_field(G, path, base + 4 * off)
-            plan.__dict__["_grad_struct"] = (base, G)
-        scs = plan.__dict__.setdefault("_scratch", {})
-        skey = (ctx.sc_bytes, dev.index)
-        scratch = scs.get(skey)
-        if scratch is None:                  # backward scratch holds nothing across calls: one buffer per size
-            scratch = scs[skey] = torch.empty(ctx.sc_bytes // 4, dtype=torch.float32, device=dev)
+        flat, G = _grad_bucket(plan, params, dev)
+        scratch = _cached_buffer(plan, "bwd", ctx.sc_bytes, dev)
         rc = lib.rd_raindrop_v2_bwd(C.byref(dims), C.byref(ctx.P), L.ptr(static), lengths.data_ptr(),
                                     node_scale.data_ptr(), ctx.ws.data_ptr(), d_logits.data_ptr(), C.byref(G),
                                     scratch.data_ptr(), L.BWD_ALL, L.stream_ptr(dev))
@@ -207,6 +192,82 @@ class RaindropV2Function(torch.autograd.Function):
             ctx.pool.append(ctx.ws)
         ctx.ws = None
         return (None, None, None, None, None, None) + tuple(grads)
+
+
+def _grad_bucket(plan, params, dev):
+    """Fresh flat gradient bucket and the rd_grads struct pointing into it (cached by base address)."""
+    layout = plan.__dict__.get("_grad_layout")
+    if layout is None:      # tightly packed flat bucket, one offset per used parameter
+        offs, total = [], 0
+        for t in params:
+            offs.append(total)
+            total += t.numel()
+        layout = plan.__dict__["_grad_layout"] = (offs, total)
+    offs, total = layout
+    flat = torch.empty(total, dtype=torch.float32, device=dev)
+    base = flat.data_ptr()
+    cachedG = plan.__dict__.get("_grad_struct")
+    if cachedG is not None and cachedG[0] == base:
+        return flat, cachedG[1]
+    G = L.RdGrads()
+    for (key, path), off in zip(plan.fields, offs):
+        _set_field(G, path, base + 4 * off)
+    plan.__dict__["_grad_struct"] = (base, G)
+    return flat, G
+
+
+def _cached_buffer(plan, name, n_bytes, dev):
+    """Device scratch that holds nothing across calls: one buffer per (name, size, device)."""
+    bufs = plan.__dict__.setdefault("_scratch", {})
+    key = (name, n_bytes, dev.index)
+    buf = bufs.get(key)
+    if buf is None:
+        buf = bufs[key] = torch.empty(max(1, n_bytes // 4), dtype=torch.float32, device=dev)
+    return buf
+
+
+def _input_grad_buffers(shape_src, static, want_in, dev):
+    """d_src / d_static / d_times tensors (None where not wanted) and the rd_input_grads struct over them."""
+    T, B, N2 = shape_src
+    f32 = dict(dtype=torch.float32, device=dev)
+    outs = (torch.empty(T, B, N2, **f32) if want_in[0] else None,
+            torch.empty(static.shape, **f32) if want_in[1] else None,
+            torch.empty(T, B, **f32) if want_in[2] else None)
+    ig = L.RdInputGrads()
+    ig.src, ig.statics, ig.times = L.ptr(outs[0]), L.ptr(outs[1]), L.ptr(outs[2])
+    return outs, ig
+
+
+def _backward_with_inputs(ctx, d_logits, want_in, want_params):
+    """RaindropV2Function.backward when an input needs a gradient or no parameter does: rd_raindrop_v2_bwd_inputs
+    (parameter gradients bit-identical to rd_raindrop_v2_bwd; none at all, and none of their launches, for a frozen
+    model)."""
+    lib = L.load()
+    plan, dims = ctx.plan, ctx.dims
+    keep, static, lengths, node_scale, _ = ctx.keep
+    dev = d_logits.device
+    flat, G = _grad_bucket(plan, keep, dev) if want_params else (None, None)
+    scratch = _cached_buffer(plan, "bwd", ctx.sc_bytes, dev)
+    in_scratch = _cached_buffer(plan, "in", lib.rd_input_grad_scratch_bytes(C.byref(dims)), dev)
+    (d_src, d_static, d_times), ig = _input_grad_buffers(ctx.src_shape, static, want_in, dev)
+    rc = lib.rd_raindrop_v2_bwd_inputs(C.byref(dims), C.byref(ctx.P), L.ptr(static), lengths.data_ptr(),
+                                       node_scale.data_ptr(), ctx.ws.data_ptr(), d_logits.data_ptr(),
+                                       C.byref(G) if G is not None else None, C.byref(ig), scratch.data_ptr(),
+                                       in_scratch.data_ptr(), L.stream_ptr(dev))
+    L.check(rc, "rd_raindrop_v2_bwd_inputs")
+    need = ctx.needs_input_grad
+    if want_params:
+        grads = torch._utils._unflatten_dense_tensors(flat, keep)
+        grads = tuple(g if n else None for g, n in zip(grads, need[6:]))
+        owner = plan.owner() if plan.owner is not None else None
+        if owner is not None:
+            owner._flat_grad = flat
+    else:
+        grads = (None,) * len(keep)
+    if not plan.debug_keep_workspace:
+        ctx.pool.append(ctx.ws)
+    ctx.ws = None
+    return (None, None, d_src, d_static, d_times, None) + grads
 
 
 class _StepSlot:
@@ -238,6 +299,7 @@ class _StepSlot:
         self.fwd_calls = self.bwd_calls = 0
         self.fwd_graph = self.bwd_graph = None
         self.pending = False          # a forward whose backward has not run yet owns the buffers
+        self.in_scratch = None
 
 
 def _run_or_capture(slot, which, fn):
@@ -283,7 +345,7 @@ class RaindropV2FlatFunction(torch.autograd.Function):
             L.check(rc, "rd_raindrop_v2_fwd")
         _run_or_capture(slot, "fwd", fwd)
         ctx.plan, ctx.slot, ctx.flat = plan, slot, flat
-        slot.pending = bool(ctx.needs_input_grad[-1])
+        slot.pending = any(ctx.needs_input_grad)
         if plan.debug_keep_workspace:
             plan.last_workspace, plan.last_dims = slot.ws, slot.dims
         return slot.logits.clone()
@@ -299,19 +361,39 @@ class RaindropV2FlatFunction(torch.autograd.Function):
             slot.scratch = torch.empty(lib.rd_backward_scratch_bytes(C.byref(slot.dims)) // 4, dtype=torch.float32,
                                        device=slot.dev)
 
-        def bwd():
-            rc = lib.rd_raindrop_v2_bwd(C.byref(slot.dims), C.byref(slot.P), L.ptr(slot.static), slot.lengths.data_ptr(),
-                                        plan.node_scale.data_ptr(), slot.ws.data_ptr(), slot.d_logits.data_ptr(),
-                                        C.byref(slot.G), slot.scratch.data_ptr(), L.BWD_ALL, L.stream_ptr(slot.dev))
-            L.check(rc, "rd_raindrop_v2_bwd")
-        _run_or_capture(slot, "bwd", bwd)
+        need = ctx.needs_input_grad
+        want_in = (need[4], need[5] and slot.static is not None, need[6])      # src, static, times
+        want_params = need[8]
+        if not any(want_in):
+            def bwd():
+                rc = lib.rd_raindrop_v2_bwd(C.byref(slot.dims), C.byref(slot.P), L.ptr(slot.static), slot.lengths.data_ptr(),
+                                            plan.node_scale.data_ptr(), slot.ws.data_ptr(), slot.d_logits.data_ptr(),
+                                            C.byref(slot.G), slot.scratch.data_ptr(), L.BWD_ALL, L.stream_ptr(slot.dev))
+                L.check(rc, "rd_raindrop_v2_bwd")
+            _run_or_capture(slot, "bwd", bwd)
+            d_in = (None, None, None)
+        else:
+            # run eagerly (not graph-captured): the forward stays one graph replay, parameter gradients are still written
+            # in place into the bucket
+            d_in, ig = _input_grad_buffers(slot.src.shape, slot.static, want_in, slot.dev)
+            if slot.in_scratch is None:
+                slot.in_scratch = torch.empty(max(1, lib.rd_input_grad_scratch_bytes(C.byref(slot.dims)) // 4),
+                                              dtype=torch.float32, device=slot.dev)
+
+            rc = lib.rd_raindrop_v2_bwd_inputs(C.byref(slot.dims), C.byref(slot.P), L.ptr(slot.static),
+                                               slot.lengths.data_ptr(), plan.node_scale.data_ptr(), slot.ws.data_ptr(),
+                                               slot.d_logits.data_ptr(), C.byref(slot.G) if want_params else None,
+                                               C.byref(ig), slot.scratch.data_ptr(), slot.in_scratch.data_ptr(),
+                                               L.stream_ptr(slot.dev))
+            L.check(rc, "rd_raindrop_v2_bwd_inputs")
         slot.pending = False
-        flat.grads_ready = True
-        owner = plan.owner() if plan.owner is not None else None
-        if owner is not None:
-            owner._flat_grad = flat.flat_g
+        if want_params:
+            flat.grads_ready = True
+            owner = plan.owner() if plan.owner is not None else None
+            if owner is not None:
+                owner._flat_grad = flat.flat_g
         # flat_p.grad already IS flat_g (written in place by the kernels): nothing for autograd to accumulate
-        return (None,) * 9
+        return (None, None, None, None) + d_in + (None, None)
 
 
 def flat_forward(plan, training, flat, src, static, times, lengths):

@@ -59,6 +59,10 @@ class RdGrads(C.Structure):
                 ("layer", RdLayer * RD_MAX_LAYERS)]
 
 
+class RdInputGrads(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("statics", C.c_void_p), ("times", C.c_void_p)]
+
+
 class RdWgradItem(C.Structure):
     _fields_ = [("d_out", C.c_void_p), ("x", C.c_void_p), ("rows", C.c_int64), ("out_features", C.c_int32),
                 ("in_features", C.c_int32), ("d_weight", C.c_void_p), ("d_bias", C.c_void_p), ("partial", C.c_void_p)]
@@ -91,6 +95,10 @@ SIGNATURES = {
     "rd_raindrop_v2_bwd": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams), C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RdGrads), C.c_void_p,
                                      C.c_int32, C.c_void_p]),
+    "rd_input_grad_scratch_bytes": (C.c_size_t, [C.POINTER(RdDims)]),
+    "rd_raindrop_v2_bwd_inputs": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.POINTER(RdGrads), C.POINTER(RdInputGrads),
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "rd_positional_encoding": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_float), C.c_int32, C.c_void_p,
                                          C.c_int64, C.c_int32, C.c_void_p]),
     "rd_encoder_head_fwd": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams)] + [C.c_void_p] * 9),
