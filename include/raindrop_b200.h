@@ -246,6 +246,14 @@ int rd_encoder_head_fwd(const rd_dims* dims, const rd_params* params, const floa
 int rd_encoder_head_bwd(const rd_dims* dims, const rd_params* params, const float* statics, const int64_t* lengths,
                         const void* workspace, const float* d_logits, const rd_grads* grads, void* scratch,
                         float* d_enc_in, void* stream);
+/* rd_encoder_head_bwd plus d_statics [B, d_static] = d(loss)/d(statics) through emb (code/models_rd.py:134,188), written,
+ * not accumulated (may be NULL; needs d_static > 0).  d_enc_in may be NULL when only d_statics is wanted.  grads == NULL:
+ * no parameter gradient is computed (frozen model, attribution): the weight-gradient GEMMs, LayerNorm column sums and
+ * head parameter outputs are skipped, and with d_enc_in also NULL the encoder layers are not visited at all.  grads !=
+ * NULL: every parameter gradient and d_enc_in are bit-identical to rd_encoder_head_bwd. */
+int rd_encoder_head_bwd_inputs(const rd_dims* dims, const rd_params* params, const float* statics, const int64_t* lengths,
+                               const void* workspace, const float* d_logits, const rd_grads* grads, float* d_enc_in,
+                               float* d_statics, void* scratch, void* stream);
 /* y[i] = x[i] * keep(site, i) / (1 - p): nn.Dropout driven by the library's counter-based stream (rng_captured =
  * {seed, counter} on the device).  The same call on a gradient is its backward. */
 int rd_dropout(const float* x, int64_t n, float p, const uint64_t* rng_captured, uint32_t site, float* y, void* stream);
@@ -255,6 +263,11 @@ int rd_dropout(const float* x, int64_t n, float p, const uint64_t* rng_captured,
  * Replaces PositionalEncodingTF.getPE (code/models_rd.py:28-37) without the host round trip. */
 int rd_positional_encoding(const float* times, int64_t n_tokens, const float* timescales_host, int32_t d_pe,
                            float* out, int64_t ld, int32_t col0, void* stream);
+/* Its backward: d_times[tok] = sum_j (d_sin_j cos_j - d_cos_j sin_j) / ts_j, from the saved encoding pe and its gradient
+ * d_pe (both laid out as `out` above: [tok*ld + col0 + 0..d_pe_width-1]; d_pe_width even, <= 64).  No trigonometry: the
+ * sin / cos columns of the forward are the derivative.  d_times [n_tokens], written, not accumulated. */
+int rd_positional_encoding_bwd(const float* pe, const float* d_pe, int64_t n_tokens, const float* timescales_host,
+                               int32_t d_pe_width, int64_t ld, int32_t col0, float* d_times, void* stream);
 
 /* out[rows, out_f] = [relu](x[rows, in_f] . weight[out_f, in_f]^T + bias): the encoder's projection
  * GEMM on its own (torch.nn.Linear inside nn.TransformerEncoderLayer, code/models_rd.py:232-237).
@@ -299,7 +312,9 @@ int rd_linear_wgrad_group(const rd_wgrad_item* items, int32_t n, void* stream);
  *   out [rows, H*F];  alpha [n_graphs, E, H] (post-softmax, as returned by the reference).
  * Backward: writes d_x (may be NULL), d_w* / d_b* (written, not accumulated; with edge_w the q/k projections take no
  * part in the output, code/transformer_conv.py:199-200, so their gradients are zeros) and d_edge_w [E] (optional,
- * only with edge_w).  scratch: rd_transformer_conv_scratch_bytes(..., backward) bytes. */
+ * only with edge_w).  The weight / bias gradient pointers may be NULL: a NULL d_w* skips that projection's weight gradient
+ * (its d_b* must then be NULL too); with all eight NULL (frozen layer) no weight-gradient launch is issued, and d_x /
+ * d_edge_w are the same as with them.  scratch: rd_transformer_conv_scratch_bytes(..., backward) bytes. */
 size_t rd_transformer_conv_scratch_bytes(int32_t n_nodes, int32_t n_graphs, int32_t in_ch, int32_t heads,
                                          int32_t out_ch, int32_t E, int32_t backward);
 int rd_transformer_conv_fwd(const float* x, int32_t n_nodes, int32_t n_graphs, int64_t node_stride,

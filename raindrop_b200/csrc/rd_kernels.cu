@@ -266,11 +266,13 @@ __global__ void lift_posenc_kernel(const float* __restrict__ src, const float* _
 //                           code/models_rd.py:290); with dX0 (CUDA-core fallback of the lift backward, already gated and
 //                           scaled) also d_src[t, b, n] = sum_k dX0[(b*N+n), t*d_ob+k] * R_u[n*d_ob+k]
 //   next n_times          : d_times[tok] = sum_j (dZ[tok, pe+j] Z[tok, pe+h+j] - dZ[tok, pe+h+j] Z[tok, pe+j]) / ts_j,
-//                           from the saved sin / cos columns of the encoder input (code/models_rd.py:33-35)
-//   next n_static         : d_static[b, i] = sum_j dfeat[b, D+j] emb_w[j, i]        (code/models_rd.py:293-294)
-__global__ void input_grad_tail_kernel(int B, int T, int N, int d_ob, int D, int pe_col, const float* __restrict__ dZ,
-                                       const float* __restrict__ Z, TS8 ts, const float* __restrict__ dfeat, int Df,
-                                       const float* __restrict__ emb_w, int ds, const float* __restrict__ dX0,
+//                           from the saved sin / cos columns (row stride pe_ld) of the encoder input
+//                           (code/models_rd.py:33-35); with n_src = n_static = 0 this is rd_positional_encoding_bwd
+//   next n_static         : d_static[b, i] = sum_{j < emb} dfeat[b, D+j] emb_w[j, i]        (code/models_rd.py:293-294)
+__global__ void input_grad_tail_kernel(int B, int T, int N, int d_ob, int D, long long pe_ld, int pe_col,
+                                       const float* __restrict__ dZ, const float* __restrict__ Z, TS8 ts,
+                                       const float* __restrict__ dfeat, int Df, const float* __restrict__ emb_w, int emb,
+                                       int ds, const float* __restrict__ dX0,
                                        const float* __restrict__ R_u, long long n_src, long long n_times,
                                        long long n_static, float* __restrict__ d_src, float* __restrict__ d_times,
                                        float* __restrict__ d_static) {
@@ -294,8 +296,8 @@ __global__ void input_grad_tail_kernel(int B, int T, int N, int d_ob, int D, int
   o -= n_src;
   if (o < n_times) {
     const int h = ts.d_pe >> 1;
-    const float* dz = dZ + o * D + pe_col;
-    const float* z = Z + o * D + pe_col;
+    const float* dz = dZ + o * pe_ld + pe_col;
+    const float* z = Z + o * pe_ld + pe_col;
     float a = 0.f;
     for (int j = 0; j < h; ++j) a += (dz[j] * z[h + j] - dz[h + j] * z[j]) / ts.v[j];
     d_times[o] = a;
@@ -306,7 +308,7 @@ __global__ void input_grad_tail_kernel(int B, int T, int N, int d_ob, int D, int
     const int b = (int)(o / ds), i = (int)(o - (long long)b * ds);
     const float* df = dfeat + (long long)b * Df + D;
     float a = 0.f;
-    for (int j = 0; j < N; ++j) a += df[j] * __ldg(emb_w + (long long)j * ds + i);
+    for (int j = 0; j < emb; ++j) a += df[j] * __ldg(emb_w + (long long)j * ds + i);
     d_static[o] = a;
   }
 }
@@ -890,23 +892,39 @@ int posenc(const float* times, int64_t n_tokens, const float* ts_host, int d_pe,
   return lift_posenc(nullptr, nullptr, 0, 0, 0, 0, 0.f, nullptr, 0, nullptr, times, n_tokens, ts_host, d_pe, out, ld, col0, st);
 }
 
-int input_grad_tail(int B, int T, int N, int d_ob, int D, const float* dZ, const float* Z, const float* ts_host,
-                    int d_pe, const float* dfeat, int Df, const float* emb_w, int ds, const float* dX0, const float* R_u,
-                    float* d_src, float* d_times, float* d_static, cudaStream_t st) {
-  if (d_pe < 2 || d_pe > 64 || (d_pe & 1)) { set_error("input_grad_tail: positional encoding width must be even and <= 64"); return -2; }
-  const int64_t n_src = d_src ? (int64_t)T * B * N : 0;
-  const int64_t n_times = d_times ? (int64_t)T * B : 0;
-  const int64_t n_static = d_static ? (int64_t)B * ds : 0;
+static int launch_input_grad_tail(int B, int T, int N, int d_ob, int D, int64_t pe_ld, int pe_col, const float* dZ,
+                                  const float* Z, const float* ts_host, int d_pe, const float* dfeat, int Df,
+                                  const float* emb_w, int emb, int ds, const float* dX0, const float* R_u, int64_t n_src,
+                                  int64_t n_times, int64_t n_static, float* d_src, float* d_times, float* d_static,
+                                  cudaStream_t st) {
+  if (d_pe < 2 || d_pe > 64 || (d_pe & 1)) { set_error("positional encoding width must be even and <= 64"); return -2; }
   TS8 ts;
   memset(&ts, 0, sizeof(ts));
   ts.d_pe = d_pe;
   memcpy(ts.v, ts_host, sizeof(float) * (d_pe / 2));
   const int64_t total = n_src + n_times + n_static;
   if (total <= 0) return 0;
-  launch_pdl(input_grad_tail_kernel, dim3(blocks_for(total)), dim3(TPB), 0, st, B, T, N, d_ob, D, D - d_pe, dZ, Z, ts, dfeat,
-             Df, emb_w, ds, dX0, R_u, (long long)n_src, (long long)n_times, (long long)n_static, d_src, d_times, d_static);
+  launch_pdl(input_grad_tail_kernel, dim3(blocks_for(total)), dim3(TPB), 0, st, B, T, N, d_ob, D, (long long)pe_ld, pe_col,
+             dZ, Z, ts, dfeat, Df, emb_w, emb, ds, dX0, R_u, (long long)n_src, (long long)n_times, (long long)n_static, d_src,
+             d_times, d_static);
   RD_CHECK_LAUNCH("input_grad_tail_kernel");
   return 0;
+}
+
+int input_grad_tail(int B, int T, int N, int d_ob, int D, const float* dZ, const float* Z, const float* ts_host,
+                    int d_pe, const float* dfeat, int Df, const float* emb_w, int emb, int ds, const float* dX0,
+                    const float* R_u, float* d_src, float* d_times, float* d_static, cudaStream_t st) {
+  const int64_t n_src = d_src ? (int64_t)T * B * N : 0;
+  const int64_t n_times = d_times ? (int64_t)T * B : 0;
+  const int64_t n_static = d_static ? (int64_t)B * ds : 0;
+  return launch_input_grad_tail(B, T, N, d_ob, D, D, D - d_pe, dZ, Z, ts_host, d_pe, dfeat, Df, emb_w, emb, ds, dX0, R_u,
+                                n_src, n_times, n_static, d_src, d_times, d_static, st);
+}
+
+int posenc_bwd(const float* pe, const float* d_pe, int64_t n_tokens, const float* ts_host, int width, int64_t ld, int col0,
+               float* d_times, cudaStream_t st) {
+  return launch_input_grad_tail(0, 0, 0, 0, 0, ld, col0, d_pe, pe, ts_host, width, nullptr, 0, nullptr, 0, 0, nullptr,
+                                nullptr, 0, n_tokens, 0, nullptr, d_times, nullptr, st);
 }
 
 int node_scale(const int64_t* edge_tgt, const float* edge_w, int E, int N, float* s, cudaStream_t st) {

@@ -93,10 +93,15 @@ int obprop_out_grad(const float* dZ, const float* Z, const float* s, int B, int 
 //   d_src [T, B, 2N]: mask half zeroed; value half from dX0 [B*N, T*d_ob] (gated, scaled: the CUDA-core fallback of the
 //                     lift backward) when dX0 != null, else left to the tensor-core store
 //   d_times [T, B]  : from dZ / Z [T, B, D] (the encoder input's last d_pe columns are sin | cos of times / ts_host[j])
-//   d_static [B, ds]: dfeat[b, D : D+N] . emb_w [N, ds]   (dfeat [B, Df] from head_bwd)
+//   d_static [B, ds]: dfeat[b, D : D+emb] . emb_w [emb, ds]   (dfeat [B, Df] from head_bwd; emb = N for Raindrop_v2,
+//                     d_model for legacy Raindrop v1)
 int input_grad_tail(int B, int T, int N, int d_ob, int D, const float* dZ, const float* Z, const float* ts_host,
-                    int d_pe, const float* dfeat, int Df, const float* emb_w, int ds, const float* dX0, const float* R_u,
-                    float* d_src, float* d_times, float* d_static, cudaStream_t st);
+                    int d_pe, const float* dfeat, int Df, const float* emb_w, int emb, int ds, const float* dX0,
+                    const float* R_u, float* d_src, float* d_times, float* d_static, cudaStream_t st);
+// d_times[tok] from the saved encoding pe and its gradient d_pe (both at [tok*ld + col0 + 0..width)): the times branch of
+// the same kernel on its own (no trigonometry: d sin = cos / ts, d cos = -sin / ts)
+int posenc_bwd(const float* pe, const float* d_pe, int64_t n_tokens, const float* ts_host, int width, int64_t ld, int col0,
+               float* d_times, cudaStream_t st);
 
 // y[i] = x[i] * mask(site, i)   (re-generates the forward's dropout mask)
 int apply_dropout(const float* x, int64_t n, float p, const uint64_t* rng, uint32_t site, float* y,

@@ -432,7 +432,10 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
   const float scale = 1.f / sqrtf((float)s.hd);
   const int64_t row3 = (int64_t)s.B * 3 * s.D;
   const int64_t TT = (int64_t)s.T * s.T;
-  for (int l = s.L - 1; l >= 0; --l) {
+  // the encoder layers are needed for parameter gradients or d(loss)/d(encoder input); a head-only call for d_statics
+  // of a frozen model (rd_encoder_head_bwd_inputs with grads = d_enc_in = NULL) stops at the head
+  const bool enc = pg || d_z0_out || (phases & RD_BWD_OBPROP);
+  for (int l = enc ? s.L - 1 : -1; l >= 0; --l) {
     const rd_encoder_layer_params& E = P->layer[l];
     const rd_encoder_layer_grads& GE = G->layer[l];
     const float* x = ws + w.Z[l];
@@ -581,7 +584,7 @@ static int raindrop_bwd(const rd_dims* dims, const rd_params* P, const float* st
   }
   if (IG && (IG->src || IG->times || IG->statics)) {
     RD_TRY(input_grad_tail(s.B, s.T, s.N, s.dob, s.D, gA, ws + w.Z[0], dims->pe_timescales, RD_D_PE, sc + b.dfeat, s.Df,
-                           P->emb_weight, s.ds, (d_src && !lift_bwd_tc(s)) ? isc + in_layout(s).dX0 : nullptr, P->R_u,
+                           P->emb_weight, s.emb, s.ds, (d_src && !lift_bwd_tc(s)) ? isc + in_layout(s).dX0 : nullptr, P->R_u,
                            IG->src, IG->times, IG->statics, st));
   }
   return 0;
@@ -830,6 +833,33 @@ int rd_encoder_head_bwd(const rd_dims* dims, const rd_params* params, const floa
   }
   return raindrop_bwd(dims, params, statics, lengths, nullptr, (const float*)workspace, d_logits, grads, (float*)scratch,
                       RD_BWD_ENCODER, d_enc_in, (cudaStream_t)stream);
+}
+
+int rd_encoder_head_bwd_inputs(const rd_dims* dims, const rd_params* params, const float* statics, const int64_t* lengths,
+                               const void* workspace, const float* d_logits, const rd_grads* grads, float* d_enc_in,
+                               float* d_statics, void* scratch, void* stream) {
+  if (!dims || !params || !lengths || !workspace || !d_logits || !scratch) {
+    set_error("rd_encoder_head_bwd_inputs: NULL argument");
+    return -2;
+  }
+  if (!grads && !d_enc_in && !d_statics) { set_error("rd_encoder_head_bwd_inputs: no gradient requested"); return -2; }
+  if (d_statics && (dims->d_static < 1 || !statics || !params->emb_weight)) {
+    set_error("rd_encoder_head_bwd_inputs: a static gradient needs d_static > 0, statics and emb_weight");
+    return -2;
+  }
+  rd_input_grads ig = {nullptr, d_statics, nullptr};
+  return raindrop_bwd(dims, params, statics, lengths, nullptr, (const float*)workspace, d_logits, grads, (float*)scratch,
+                      RD_BWD_ENCODER, d_enc_in, (cudaStream_t)stream, d_statics ? &ig : nullptr);
+}
+
+int rd_positional_encoding_bwd(const float* pe, const float* d_pe, int64_t n_tokens, const float* timescales_host,
+                               int32_t d_pe_width, int64_t ld, int32_t col0, float* d_times, void* stream) {
+  if (!pe || !d_pe || !timescales_host || !d_times || n_tokens < 0 || col0 < 0 || ld < (int64_t)col0 + d_pe_width) {
+    set_error("rd_positional_encoding_bwd: bad arguments");
+    return -2;
+  }
+  if (n_tokens == 0) return 0;
+  return posenc_bwd(pe, d_pe, n_tokens, timescales_host, d_pe_width, ld, col0, d_times, (cudaStream_t)stream);
 }
 
 int rd_dropout(const float* x, int64_t n, float p, const uint64_t* rng_captured, uint32_t site, float* y, void* stream) {

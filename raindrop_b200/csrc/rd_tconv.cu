@@ -246,7 +246,8 @@ extern "C" int rd_transformer_conv_fwd(const float* x, int32_t n_nodes, int32_t 
 
 // d_x (may be NULL), d_w*/d_b* [HF, in] / [HF] (written, not accumulated), d_edge_w [E] (only with edge_w, may be NULL).
 // With edge_w given, lin_query / lin_key take no part in the output (code/transformer_conv.py:199-200): their
-// gradients are written as zeros.
+// gradients are written as zeros.  A NULL d_w* skips that projection's weight gradient (its d_b* must be NULL too); with
+// all eight NULL (frozen layer) no weight-gradient launch is issued and d_x / d_edge_w are computed as before.
 extern "C" int rd_transformer_conv_bwd(const float* x, int32_t n_nodes, int32_t n_graphs, int64_t node_stride,
                                        int64_t graph_stride, int32_t in_ch, int32_t heads, int32_t out_ch,
                                        const int64_t* edge_src, const int64_t* edge_tgt, const float* edge_w, int32_t E,
@@ -256,8 +257,12 @@ extern "C" int rd_transformer_conv_bwd(const float* x, int32_t n_nodes, int32_t 
                                        float* d_ws, float* d_bs, float* d_edge_w, void* scratch, void* stream) {
   RD_TRY(check_common("rd_transformer_conv_bwd", x, edge_src, edge_tgt, n_nodes, n_graphs, in_ch, heads, out_ch, E, node_stride,
                       graph_stride));
-  if (!wq || !wk || !wv || !ws || !alpha || !d_out || !d_wq || !d_bq || !d_wk || !d_bk || !d_wv || !d_bv || !d_ws || !d_bs || !scratch) {
+  if (!wq || !wk || !wv || !ws || !alpha || !d_out || !scratch) {
     set_error("rd_transformer_conv_bwd: NULL argument");
+    return -2;
+  }
+  if ((!d_wq && d_bq) || (!d_wk && d_bk) || (!d_wv && d_bv) || (!d_ws && d_bs)) {
+    set_error("rd_transformer_conv_bwd: a bias gradient needs its weight gradient");
     return -2;
   }
   cudaStream_t st = (cudaStream_t)stream;
@@ -274,12 +279,13 @@ extern "C" int rd_transformer_conv_bwd(const float* x, int32_t n_nodes, int32_t 
   }
   RD_TRY(gemm(proj(x, in_ch, wv, bv, v, l.rows, HF), st));
   // skip term: out = ... + x Ws^T + bs
-  RD_TRY(wgrad(d_out, HF, x, in_ch, l.rows, d_ws, d_bs, partial, st));
+  if (d_ws) RD_TRY(wgrad(d_out, HF, x, in_ch, l.rows, d_ws, d_bs, partial, st));
   if (d_x) RD_TRY(gemm(back(d_out, HF, ws, in_ch, d_x, l.rows, false), st));
   const size_t wbytes = sizeof(float) * (size_t)HF * in_ch, bbytes = sizeof(float) * (size_t)HF;
+  auto zero = [&](float* p, size_t n) { if (p) cudaMemsetAsync(p, 0, n, st); };
   if (E == 0) {
-    cudaMemsetAsync(d_wq, 0, wbytes, st); cudaMemsetAsync(d_wk, 0, wbytes, st); cudaMemsetAsync(d_wv, 0, wbytes, st);
-    cudaMemsetAsync(d_bq, 0, bbytes, st); cudaMemsetAsync(d_bk, 0, bbytes, st); cudaMemsetAsync(d_bv, 0, bbytes, st);
+    zero(d_wq, wbytes); zero(d_wk, wbytes); zero(d_wv, wbytes);
+    zero(d_bq, bbytes); zero(d_bk, bbytes); zero(d_bv, bbytes);
     return 0;
   }
   TcP p{n_nodes, n_graphs, heads, out_ch, E, node_stride, graph_stride, edge_src, edge_tgt};
@@ -288,20 +294,20 @@ extern "C" int rd_transformer_conv_bwd(const float* x, int32_t n_nodes, int32_t 
   RD_CHECK_LAUNCH("tconv_bwd_softmax_kernel");
   tconv_bwd_src_kernel<<<dim3(n_nodes, n_graphs), 128, 0, st>>>(p, q, alpha, dlogit, d_out, dv, qk ? dk : nullptr);
   RD_CHECK_LAUNCH("tconv_bwd_src_kernel");
-  RD_TRY(wgrad(dv, HF, x, in_ch, l.rows, d_wv, d_bv, partial, st));
+  if (d_wv) RD_TRY(wgrad(dv, HF, x, in_ch, l.rows, d_wv, d_bv, partial, st));
   if (d_x) RD_TRY(gemm(back(dv, HF, wv, in_ch, d_x, l.rows, true), st));
   if (qk) {
     tconv_bwd_tgt_kernel<<<dim3(n_nodes, n_graphs), 128, 0, st>>>(p, k, dlogit, dq);
     RD_CHECK_LAUNCH("tconv_bwd_tgt_kernel");
-    RD_TRY(wgrad(dq, HF, x, in_ch, l.rows, d_wq, d_bq, partial, st));
-    RD_TRY(wgrad(dk, HF, x, in_ch, l.rows, d_wk, d_bk, partial, st));
+    if (d_wq) RD_TRY(wgrad(dq, HF, x, in_ch, l.rows, d_wq, d_bq, partial, st));
+    if (d_wk) RD_TRY(wgrad(dk, HF, x, in_ch, l.rows, d_wk, d_bk, partial, st));
     if (d_x) {
       RD_TRY(gemm(back(dq, HF, wq, in_ch, d_x, l.rows, true), st));
       RD_TRY(gemm(back(dk, HF, wk, in_ch, d_x, l.rows, true), st));
     }
   } else {
-    cudaMemsetAsync(d_wq, 0, wbytes, st); cudaMemsetAsync(d_wk, 0, wbytes, st);
-    cudaMemsetAsync(d_bq, 0, bbytes, st); cudaMemsetAsync(d_bk, 0, bbytes, st);
+    zero(d_wq, wbytes); zero(d_wk, wbytes);
+    zero(d_bq, bbytes); zero(d_bk, bbytes);
     if (d_edge_w) {
       tconv_bwd_edgew_kernel<<<(unsigned)ceil_div(E, 256), 256, 0, st>>>(p, dlogit, d_edge_w);
       RD_CHECK_LAUNCH("tconv_bwd_edgew_kernel");

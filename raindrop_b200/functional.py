@@ -525,15 +525,43 @@ def node_scale(edge_index, edge_weights, n_nodes):
     return s
 
 
+def _pe_timescales_c(max_len, d_pe):
+    return (C.c_float * (d_pe // 2))(*[float(v) for v in pe_timescales(max_len, d_pe)])
+
+
 def positional_encoding(times, max_len, d_pe=16):
-    """[T, B] -> [T, B, d_pe] on the device (rd_positional_encoding); d_pe even, <= 64."""
+    """[T, B] -> [T, B, d_pe] on the device (rd_positional_encoding); d_pe even, <= 64.  No autograd node: see
+    PositionalEncodingFunction for the differentiable version."""
     lib = L.load()
     t = _as_f32(times)
     out = torch.empty(t.shape + (d_pe,), dtype=torch.float32, device=t.device)
-    ts = (C.c_float * (d_pe // 2))(*[float(v) for v in pe_timescales(max_len, d_pe)])
-    L.check(lib.rd_positional_encoding(t.data_ptr(), t.numel(), ts, d_pe, out.data_ptr(), d_pe, 0, L.stream_ptr(t.device)),
-            "rd_positional_encoding")
+    L.check(lib.rd_positional_encoding(t.data_ptr(), t.numel(), _pe_timescales_c(max_len, d_pe), d_pe, out.data_ptr(), d_pe, 0,
+                                       L.stream_ptr(t.device)), "rd_positional_encoding")
     return out
+
+
+class PositionalEncodingFunction(torch.autograd.Function):
+    """pe = [sin(times / ts), cos(times / ts)] (code/models_rd.py:28-37) with d(pe)/d(times): the forward is
+    positional_encoding; the backward (rd_positional_encoding_bwd) forms d_times from the saved sin / cos columns."""
+
+    @staticmethod
+    def forward(ctx, times, max_len, d_pe):
+        pe = positional_encoding(times, max_len, d_pe)
+        ctx.max_len, ctx.d_pe, ctx.shape = max_len, d_pe, times.shape
+        ctx.save_for_backward(pe)
+        return pe
+
+    @staticmethod
+    def backward(ctx, d_pe):
+        lib = L.load()
+        (pe,) = ctx.saved_tensors
+        d_pe = _as_f32(d_pe)
+        d_times = torch.empty(ctx.shape, dtype=torch.float32, device=pe.device)
+        n = d_times.numel()
+        L.check(lib.rd_positional_encoding_bwd(pe.data_ptr(), d_pe.data_ptr(), n, _pe_timescales_c(ctx.max_len, ctx.d_pe),
+                                               ctx.d_pe, ctx.d_pe, 0, d_times.data_ptr(), L.stream_ptr(pe.device)),
+                "rd_positional_encoding_bwd")
+        return d_times, None, None
 
 
 def linear(x, weight, bias=None, relu=False):
@@ -591,17 +619,20 @@ class TransformerConvFunction(torch.autograd.Function):
         d_out = _as_f32(d_out)
         dev = x.device
         d_x = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-        gw = [torch.empty(heads * F_, in_ch, dtype=torch.float32, device=dev) for _ in range(4)]
-        gb = [torch.empty(heads * F_, dtype=torch.float32, device=dev) for _ in range(4)]
+        if any(ctx.needs_input_grad[6:]):
+            gw = [torch.empty(heads * F_, in_ch, dtype=torch.float32, device=dev) for _ in range(4)]
+            gb = [torch.empty(heads * F_, dtype=torch.float32, device=dev) for _ in range(4)]
+        else:       # frozen layer: NULL weight / bias gradients, no weight-gradient launch
+            gw, gb = [None] * 4, [None] * 4
         d_ew = torch.zeros(E, dtype=torch.float32, device=dev) if (ctx.ew is not None and ctx.needs_input_grad[2]) else None
         sc = torch.empty(max(1, lib.rd_transformer_conv_scratch_bytes(n_nodes, n_graphs, in_ch, heads, F_, E, 1) // 4),
                          dtype=torch.float32, device=dev)
         rc = lib.rd_transformer_conv_bwd(x.data_ptr(), n_nodes, n_graphs, node_stride, graph_stride, in_ch, heads, F_,
                                          src_i.data_ptr(), tgt_i.data_ptr(), L.ptr(ctx.ew), E, wq.data_ptr(), bq.data_ptr(),
                                          wk.data_ptr(), bk.data_ptr(), wv.data_ptr(), bv.data_ptr(), ws.data_ptr(),
-                                         alpha.data_ptr(), d_out.data_ptr(), L.ptr(d_x), gw[0].data_ptr(), gb[0].data_ptr(),
-                                         gw[1].data_ptr(), gb[1].data_ptr(), gw[2].data_ptr(), gb[2].data_ptr(), gw[3].data_ptr(),
-                                         gb[3].data_ptr(), L.ptr(d_ew), sc.data_ptr(), L.stream_ptr(dev))
+                                         alpha.data_ptr(), d_out.data_ptr(), L.ptr(d_x), L.ptr(gw[0]), L.ptr(gb[0]),
+                                         L.ptr(gw[1]), L.ptr(gb[1]), L.ptr(gw[2]), L.ptr(gb[2]), L.ptr(gw[3]),
+                                         L.ptr(gb[3]), L.ptr(d_ew), sc.data_ptr(), L.stream_ptr(dev))
         L.check(rc, "rd_transformer_conv_bwd")
         return (d_x, None, d_ew, None, None, None, gw[0], gb[0], gw[1], gb[1], gw[2], gb[2], gw[3], gb[3])
 
@@ -632,6 +663,8 @@ class LinearFunction(torch.autograd.Function):
         x, weight = ctx.saved_tensors
         dy = _as_f32(dy)
         dx = linear(dy, weight.t().contiguous()) if ctx.needs_input_grad[0] else None
+        if not (ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2])):
+            return dx, None, None           # frozen layer: no weight-gradient launch
         rows, out_f = dy.shape
         in_f = x.shape[1]
         dW = torch.empty_like(weight)
@@ -703,22 +736,38 @@ class EncoderHeadFunction(torch.autograd.Function):
         keep, static, lengths = ctx.keep
         d_logits = _as_f32(d_logits)
         dev = d_logits.device
-        offs, total = [], 0
-        for t in keep:
-            offs.append(total)
-            total += t.numel()
-        flat = torch.empty(total, dtype=torch.float32, device=dev)
-        G = L.RdGrads()
-        for (key, path), off in zip(plan.fields, offs):
-            _set_field(G, path, flat.data_ptr() + 4 * off)
+        need = ctx.needs_input_grad
+        want_static = need[3] and static is not None
+        want_params = any(need[5:])
+        flat, G = None, None
+        if want_params:
+            offs, total = [], 0
+            for t in keep:
+                offs.append(total)
+                total += t.numel()
+            flat = torch.empty(total, dtype=torch.float32, device=dev)
+            G = L.RdGrads()
+            for (key, path), off in zip(plan.fields, offs):
+                _set_field(G, path, flat.data_ptr() + 4 * off)
         sc = torch.empty(lib.rd_backward_scratch_bytes(C.byref(dims)) // 4, dtype=torch.float32, device=dev)
-        dz = torch.empty(ctx.shape, dtype=torch.float32, device=dev)
-        rc = lib.rd_encoder_head_bwd(C.byref(dims), C.byref(ctx.P), L.ptr(static), lengths.data_ptr(), ctx.ws.data_ptr(),
-                                     d_logits.data_ptr(), C.byref(G), sc.data_ptr(), dz.data_ptr(), L.stream_ptr(dev))
-        L.check(rc, "rd_encoder_head_bwd")
-        grads = torch._utils._unflatten_dense_tensors(flat, keep)
+        dz = torch.empty(ctx.shape, dtype=torch.float32, device=dev) if (need[2] or not want_static) else None
+        d_static = torch.empty(static.shape, dtype=torch.float32, device=dev) if want_static else None
+        if want_params and not want_static:
+            rc = lib.rd_encoder_head_bwd(C.byref(dims), C.byref(ctx.P), L.ptr(static), lengths.data_ptr(), ctx.ws.data_ptr(),
+                                         d_logits.data_ptr(), C.byref(G), sc.data_ptr(), dz.data_ptr(), L.stream_ptr(dev))
+            L.check(rc, "rd_encoder_head_bwd")
+        else:
+            rc = lib.rd_encoder_head_bwd_inputs(C.byref(dims), C.byref(ctx.P), L.ptr(static), lengths.data_ptr(),
+                                                ctx.ws.data_ptr(), d_logits.data_ptr(), C.byref(G) if G is not None else None,
+                                                L.ptr(dz), L.ptr(d_static), sc.data_ptr(), L.stream_ptr(dev))
+            L.check(rc, "rd_encoder_head_bwd_inputs")
+        if want_params:
+            grads = torch._utils._unflatten_dense_tensors(flat, keep)
+            grads = tuple(g if n else None for g, n in zip(grads, need[5:]))
+        else:
+            grads = (None,) * len(keep)
         ctx.ws = None
-        return (None, None, dz, None, None) + tuple(grads)
+        return (None, None, dz if need[2] else None, d_static, None) + grads
 
 
 def workspace_view(plan, which):

@@ -101,9 +101,13 @@ SIGNATURES = {
                                             C.c_void_p, C.c_void_p, C.c_void_p]),
     "rd_positional_encoding": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_float), C.c_int32, C.c_void_p,
                                          C.c_int64, C.c_int32, C.c_void_p]),
+    "rd_positional_encoding_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_float), C.c_int32, C.c_int64,
+                                             C.c_int32, C.c_void_p, C.c_void_p]),
     "rd_encoder_head_fwd": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams)] + [C.c_void_p] * 9),
     "rd_encoder_head_bwd": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.POINTER(RdGrads), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rd_encoder_head_bwd_inputs": (C.c_int, [C.POINTER(RdDims), C.POINTER(RdParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.POINTER(RdGrads), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rd_dropout": (C.c_int, [C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
     "rd_linear_scratch_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "rd_linear_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32,

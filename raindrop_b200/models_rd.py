@@ -37,7 +37,8 @@ def _device_of(*tensors):
 
 class PositionalEncodingTF(nn.Module):
     """code/models_rd.py:20-43.  The reference builds the encoding on the host with numpy and
-    copies it to the GPU (two syncs per forward); here it is one kernel on the device."""
+    copies it to the GPU (two syncs per forward); here it is one kernel on the device.  Differentiable with respect
+    to P_time, as the reference's torch ops are (RF.PositionalEncodingFunction)."""
 
     def __init__(self, d_model, max_len=500, MAX=10000):
         super().__init__()
@@ -48,7 +49,7 @@ class PositionalEncodingTF(nn.Module):
 
     def getPE(self, P_time):
         dev = _device_of(P_time)
-        return RF.positional_encoding(P_time.to(dev), self.max_len, self.d_model)
+        return RF.PositionalEncodingFunction.apply(P_time.to(dev), self.max_len, self.d_model)
 
     def forward(self, P_time):
         return self.getPE(P_time)
@@ -306,7 +307,8 @@ class Raindrop(nn.Module):
       cat positional encoding (d_pe = 36), nn.TransformerEncoder, masked mean / (lengths + 1), cat emb(static),
       mlp_static (:168-189)                                               rd_encoder_head_fwd/_bwd (the Raindrop_v2 kernels)
     `distance` = mean pairwise distance of the per-sample attention vectors (:165-166): the edge weights are shared by
-    all samples, so it is 0 -- evaluated from the returned alphas, not assumed."""
+    all samples, so it is 0 -- evaluated from the returned alphas, not assumed.
+    Autograd reaches src, static, times and a global_structure that requires grad, as in the reference (:131-166)."""
 
     def __init__(self, d_inp=36, d_model=64, nhead=4, nhid=128, nlayers=2, dropout=0.3, max_len=215, d_static=9,
                  MAX=100, perc=0.5, aggreg='mean', n_classes=2, global_structure=None):
@@ -366,9 +368,11 @@ class Raindrop(nn.Module):
         gs = self.global_structure
         if gs is None:
             raise ValueError("Raindrop v1 needs global_structure (code/models_rd.py:148)")
-        adj = gs.detach().to(device=device, dtype=torch.float32).clone()
-        adj[torch.arange(36, device=device), torch.arange(36, device=device)] = 1                   # :149
-        edge_index = torch.nonzero(adj).T.contiguous()
+        # the edge weights stay differentiable w.r.t. global_structure; the diagonal is forced to 1 out of place, so it
+        # gets zero gradient as under the reference's in-place write (:149); edge_index is data
+        eye = torch.eye(36, dtype=torch.bool, device=device)
+        adj = torch.where(eye, 1.0, gs.to(device=device, dtype=torch.float32))                        # :149
+        edge_index = torch.nonzero(adj.detach()).T.contiguous()
         edge_weights = adj[edge_index[0], edge_index[1]].contiguous()
         out, alpha = self.transconv.forward_batched(x.view(T, B, self.d_inp), edge_index, edge_weights)   # :155-166
         alpha_all = alpha[:, :, 0]                                                                    # [B, E]
